@@ -6,7 +6,7 @@ background estimation over 300 synthetic 1080p frames.  A "step" is one pass
 of the exact temporal median over the whole clip (1.87 GB, far larger than the
 126 MB L2, so every step streams from HBM).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` = frames/s with the clip resident in
 HBM; `e2e` = the same through the public numpy-style API with the clip in pinned
@@ -49,6 +49,21 @@ KERNELS = {
                           "median_kernel fix-up; algorithmic bytes / time of the three launches",
 }
 FALLBACK_HBM_GBS = 6650.0
+DUMP_BYTES = 64 * 10**6   # cap of what --dump-outputs writes
+
+
+def dump_outputs(path, background):
+    """--dump-outputs: the background the timed path returned in its last step, as float32 `background.npy` under
+    `path`, with the image rows it holds in `background_rows.npy`: every row, or a fixed seeded sample of them when
+    the whole image would exceed DUMP_BYTES."""
+    h = background.shape[0]
+    row_bytes = background[0].size * 4 + 8
+    rows = np.arange(h)
+    if h * row_bytes > DUMP_BYTES - 1024:   # 1024: room for the two .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(h, (DUMP_BYTES - 1024) // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "background.npy"), background[rows].astype(np.float32))
+    np.save(os.path.join(path, "background_rows.npy"), rows.astype(np.float64))
 
 
 def measured_peak():
@@ -336,6 +351,8 @@ def run_gpu_arm(args, wl):
     want = ((s[(n - 1) // 2] + s[n // 2]) >> 1).to(torch.uint8)
     if not torch.equal(out[h // 2:h // 2 + 4], want):
         raise SystemExit("bench: temporal median output failed its spot check")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out.cpu().numpy())   # before the worst-case block below overwrites `out`
 
     # ---- e2e: public API, clip in pinned host memory, result read back to the host ----
     e2e = None
@@ -466,7 +483,7 @@ def run_gpu_arm(args, wl):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 3 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="median_1080p", choices=sorted(WORKLOADS))
@@ -475,13 +492,23 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--configs", default="all", help="'all', 'none' or a comma list of tools/bench_configs.py workloads for the `configs` block")
     ap.add_argument("--config-steps", type=int, default=10, help="timed steps per workload of the `configs` block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the background of the last timed step to DIR/background.npy "
+                    "(float32; rank 0's clip under torchrun)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm times a separate, reduced-height clip (synth_clip_host): nothing comparable to dump
+        ap.error("--dump-outputs applies to the GPU arm only")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
-        # bounded: each step is a sample of the workload; keep the whole run to a few minutes
-        args.steps_ref = max(1, min(args.steps, 3))
+        # each step is a bounded sample of the workload (--sample-rows rows of every frame); by default 3 of them,
+        # which keeps the whole run to a few minutes
+        args.steps_ref = 3 if args.steps is None else args.steps
         args.warmup_ref = 1 if args.warmup > 0 else 0
         return run_reference_arm(args, wl)
+    if args.steps is None:
+        args.steps = 200
     return run_gpu_arm(args, wl)
 
 

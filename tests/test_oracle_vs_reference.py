@@ -1,85 +1,147 @@
-"""Oracle == the live, unmodified reference, on fresh seeded inputs (other than the committed golden fixtures).
+"""Oracle == the live, unmodified reference, on seeded inputs other than the committed golden fixtures.
 
-Runs only where the reference checkout exists (the build container: /root/reference); skipped on the GPU box.
-The reference is imported under the non-invasive shim of tests/golden/make_golden.py (stub mmcv / matplotlib,
-restore np.float / np.int).  This is what pins the oracle beyond the fixtures: different sizes, seeds and parameters
-every time the file is edited, no stored outputs."""
+With the environment variable UNSCREEN_REFERENCE naming a checkout of AnyiRao/video_unscreen, every output of the oracle
+is compared with the reference's own (imported under the non-invasive shim of tests/golden/make_golden.py: stub mmcv /
+matplotlib, restore np.float / np.int), with the tolerances written beside each call.
+
+Without it, the same oracle outputs are compared with tests/golden/oracle_pins.json: shape, dtype and the SHA-256 of
+the bytes of every integer output, and 256 seeded samples of every float64 output (checked to the tolerance used against
+the reference: scipy's spsolve may differ in the last bits between machines).  Those pins are the
+ORACLE's outputs on these inputs, not the reference's: they were recorded without a copy of the reference at hand, from
+the oracle as it stood when these tests were last changed to run against it.  They keep these extra sizes, seeds and
+parameters from drifting on every checkout.  Re-record them (ORACLE_PINS_WRITE=1 python -m pytest
+tests/test_oracle_vs_reference.py) only from an oracle that passes against the reference, with UNSCREEN_REFERENCE set so
+that the same run checks it."""
+import hashlib
+import json
 import os
 import sys
 
 import numpy as np
 import pytest
 
-REF_ROOT = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF_ROOT, "unscreen")), reason="reference checkout not present")
+REF_ROOT = os.environ.get("UNSCREEN_REFERENCE", "")
+HAVE_REF = bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "unscreen"))
+PINS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "oracle_pins.json")
+sys.path.insert(0, os.path.dirname(PINS))   # make_golden: the input generators shared with the golden fixtures
 
 from oracle import refport as R  # noqa: E402
 
 
 @pytest.fixture(scope="module")
 def ref():
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+    """the reference's modules, or None without a checkout"""
+    if not HAVE_REF:
+        return None
     from make_golden import load_reference
     U, CF, TA, BA = load_reference(REF_ROOT)
 
     class Ref:
         pass
     r = Ref()
-    r.U, r.CF, r.TA = U, CF, TA
+    r.U, r.CF, r.TA, r.BA = U, CF, TA, BA
     return r
 
 
-def test_morphology_and_counts(ref):
+def equal(a, b):
+    return np.array_equal(np.asarray(a), np.asarray(b))
+
+
+def within(tol):
+    return lambda a, b: np.abs(np.asarray(a).astype(np.float64) - np.asarray(b).astype(np.float64)).max() <= tol
+
+
+def pin_of(a):
+    p = {"shape": list(a.shape), "dtype": str(a.dtype)}
+    if a.dtype.kind == "f":
+        p["sample"] = a.reshape(-1)[np.random.default_rng(0).choice(a.size, min(a.size, 256), replace=False)].tolist()
+    else:
+        p["sha256"] = hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+    return p
+
+
+@pytest.fixture(scope="module")
+def check(ref):
+    """check(key, got, want, agree=equal): the oracle's `got` against the reference's `want()` (agree(got, want()) must
+    hold), or, without the reference, against the pin of the oracle's output `key` (see the module docstring)"""
+    write = bool(os.environ.get("ORACLE_PINS_WRITE"))
+    pins = json.load(open(PINS)) if os.path.exists(PINS) else {}
+
+    def run(key, got, want, agree=equal):
+        got = np.asarray(got)
+        if ref is not None:
+            assert agree(got, want()), key
+        elif not write:
+            assert key in pins, f"{key} has no pinned oracle output"
+            have, want_pin = pin_of(got), pins[key]
+            if "sample" in want_pin:
+                assert have["shape"] == want_pin["shape"] and have["dtype"] == want_pin["dtype"], key
+                assert agree(np.array(have["sample"]), np.array(want_pin["sample"])), key
+            else:
+                assert have == want_pin, key
+        if write:
+            pins[key] = pin_of(got)
+    yield run
+    if write:
+        with open(PINS, "w") as f:
+            f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(v)}" for k, v in sorted(pins.items())) + "\n}\n")
+
+
+def test_morphology_and_counts(ref, check):
     rng = np.random.default_rng(77)
     m = rng.integers(0, 256, (61, 83), dtype=np.uint8)
     for k, n in [(3, 1), (3, 4), (4, 1), (4, 3), (5, 2), (7, 3)]:
-        assert np.array_equal(R.dilate_mask(m, k, n), ref.U.dilate_mask(m, k, n)), (k, n)
-        assert np.array_equal(R.erode_mask(m, k, n), ref.U.erode_mask(m, k, n)), (k, n)
-    assert np.array_equal(R.get_outer_boundary(m), ref.U.get_outer_boundary(m))
+        check(f"dilate_{k}_{n}", R.dilate_mask(m, k, n), lambda: ref.U.dilate_mask(m, k, n))
+        check(f"erode_{k}_{n}", R.erode_mask(m, k, n), lambda: ref.U.erode_mask(m, k, n))
+    check("outer_boundary", R.get_outer_boundary(m), lambda: ref.U.get_outer_boundary(m))
     for t in (0.0, 0.3, 0.5, 0.9):
-        assert R.exist_foreground(m, t) == ref.U.exist_foreground(m, t)
+        check(f"exist_fg_{t}", R.exist_foreground(m, t), lambda: ref.U.exist_foreground(m, t))
 
 
-def test_inrange_and_sizes(ref):
+def test_inrange_and_sizes(ref, check):
     rng = np.random.default_rng(78)
     img = rng.integers(0, 256, (70, 94, 3), dtype=np.uint8)
     bgi = np.clip(img.astype(np.int16) + rng.integers(-25, 26, img.shape), 0, 255).astype(np.uint8)
     for col, win in [((30, 180, 60), (10, 100, 180)), ((250, 3, 7), (40, 40, 40)), ((0, 0, 0), (255, 255, 255))]:
         c = np.array(col, np.uint8)
-        assert np.array_equal(R.is_pixel_inrange(img, c, win), ref.U.is_pixel_inrange(img, c, win))
-    assert np.array_equal(R.is_pixel_inrange(img, bgi, (20, 30, 90)), ref.U.is_pixel_inrange(img, bgi, (20, 30, 90)))
+        check(f"inrange_{col[0]}_{col[1]}_{col[2]}", R.is_pixel_inrange(img, c, win), lambda: ref.U.is_pixel_inrange(img, c, win))
+    check("inrange_image", R.is_pixel_inrange(img, bgi, (20, 30, 90)), lambda: ref.U.is_pixel_inrange(img, bgi, (20, 30, 90)))
     for h, w, L in [(1080, 1920, 960), (2160, 3840, 960), (607, 411, 300), (100, 100, 37)]:
-        assert tuple(R.get_target_size(h, w, L)) == tuple(ref.U.get_target_size(h, w, L))
+        check(f"target_size_{h}_{w}_{L}", tuple(R.get_target_size(h, w, L)), lambda: tuple(ref.U.get_target_size(h, w, L)))
 
 
 @pytest.mark.parametrize("h,w,L", [(96, 160, 80), (150, 110, 60), (128, 256, 64)])
-def test_trimap(ref, h, w, L):
+def test_trimap(ref, check, h, w, L):
     rng = np.random.default_rng(h + w)
     yy, xx = np.mgrid[0:h, 0:w]
     mask = ((((xx - w / 2) / (w * 0.3)) ** 2 + ((yy - h / 2) / (h * 0.35)) ** 2) <= 1).astype(np.uint8) * 255
     mask[rng.random((h, w)) < 0.01] = 200
-    agent = ref.TA(input_long_side=L)
-    assert np.array_equal(R.generate_trimap(mask, L), agent.forward(mask.copy()))
+    agent = ref.TA(input_long_side=L) if ref else None
+    check(f"trimap_{h}_{w}_{L}", R.generate_trimap(mask, L), lambda: agent.forward(mask.copy()))
     img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
     img[mask == 0] = (60, 200, 40)
     for bg in (np.array([60, 200, 40], np.uint8), np.array([10, 10, 200], np.uint8)):
-        assert np.array_equal(R.generate_trimap_withbg(mask, img, bg, L), agent.forward(mask.copy(), img.copy(), bg.copy()))
+        check(f"trimap_{h}_{w}_{L}_bg{bg[2]}", R.generate_trimap_withbg(mask, img, bg, L),
+              lambda: agent.forward(mask.copy(), img.copy(), bg.copy()))
 
 
-def test_compositing(ref):
+def test_compositing(ref, check):
     rng = np.random.default_rng(79)
     h, w = 64, 96
     fr = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
     bg = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
     al = rng.integers(0, 256, (h, w), dtype=np.uint8)
-    assert np.abs(R.get_fg(fr, al, bg).astype(int) - ref.U.get_fg(fr.copy(), al.copy(), bg.copy()).astype(int)).max() <= 1     # cv2's HSV2BGR
-    assert np.abs(R.get_bg(al, bg).astype(int) - ref.U.get_bg(al.copy(), bg.copy()).astype(int)).max() <= 1
-    assert np.array_equal(R.get_fg_naive(fr, al), ref.U.get_fg_naive(fr.copy(), al.copy()))
-    assert np.array_equal(R.fuse_fgbg(fr, bg, al), ref.U.fuse_fgbg(fr.copy(), bg.copy(), al.copy()))
-    assert np.array_equal(R.composite_fgbg(fr, al, bg), ref.U.composite_fgbg(fr.copy(), al.copy(), bg.copy()))
+    check("get_fg", R.get_fg(fr, al, bg), lambda: ref.U.get_fg(fr.copy(), al.copy(), bg.copy()), within(1))     # cv2's HSV2BGR
+    check("get_bg", R.get_bg(al, bg), lambda: ref.U.get_bg(al.copy(), bg.copy()), within(1))
+    check("get_fg_naive", R.get_fg_naive(fr, al), lambda: ref.U.get_fg_naive(fr.copy(), al.copy()))
+    check("fuse_fgbg", R.fuse_fgbg(fr, bg, al), lambda: ref.U.fuse_fgbg(fr.copy(), bg.copy(), al.copy()))
+    check("composite_fgbg", R.composite_fgbg(fr, al, bg), lambda: ref.U.composite_fgbg(fr.copy(), al.copy(), bg.copy()))
 
 
 def test_colorfilter_predict(ref):
+    """the mixtures are fitted by the reference itself (sklearn under its own seeding): nothing to pin without it"""
+    if ref is None:
+        pytest.skip("reference checkout not present (set UNSCREEN_REFERENCE)")
     from video_unscreen_b200 import synth
     frame, seg = synth.green_frame(180, 320, t=2, n=10, seed=9)
     agent = ref.CF(input_long_side=160)
@@ -93,7 +155,7 @@ def test_colorfilter_predict(ref):
     assert np.abs(bg.astype(int) - bg_ref.astype(int)).max() <= 1
 
 
-def test_replace_geometry(ref):
+def test_replace_geometry(ref, check):
     """shift_fg (bit-exact) and rescale_fg (the documented tie tolerance against cv2's IPP cubic) of the live reference,
     and the composed frame of tools/replace/replace.py:69-76."""
     rng = np.random.default_rng(81)
@@ -101,22 +163,27 @@ def test_replace_geometry(ref):
     m3 = np.repeat(rng.integers(0, 256, (108, 192, 1), dtype=np.uint8), 3, axis=2)
     bg = rng.integers(0, 256, (108, 192, 3), dtype=np.uint8)
     for dx, dy in [(3, -2), (0.5, 0.5), (-6.37, 2.81)]:
-        assert np.array_equal(R.shift_fg(fg, dx, dy), ref.U.shift_fg(fg, dx=dx, dy=dy))
-        assert np.array_equal(R.shift_fg(m3[..., 0], dx, dy), ref.U.shift_fg(m3[..., 0], dx=dx, dy=dy))
+        check(f"shift_{dx}_{dy}", R.shift_fg(fg, dx, dy), lambda: ref.U.shift_fg(fg, dx=dx, dy=dy))
+        check(f"shift_mask_{dx}_{dy}", R.shift_fg(m3[..., 0], dx, dy), lambda: ref.U.shift_fg(m3[..., 0], dx=dx, dy=dy))
+
+    def ties(tol, frac):
+        def agree(a, b):
+            d = np.abs(a.astype(int) - b.astype(int))
+            return d.max() <= tol and (d > 0).mean() <= frac
+        return agree
     for sc in (1.2, 1.1):
-        d = np.abs(R.rescale_fg(fg, sc).astype(int) - ref.U.rescale_fg(fg, scale_factor=sc).astype(int))
-        assert d.max() <= 1 and (d > 0).mean() <= 1e-4
-    # replace.py:69-76 restated with the reference's own functions
-    f = ref.U.rescale_fg(ref.U.shift_fg(fg, dx=3, dy=-2), scale_factor=1.2)
-    m = ref.U.rescale_fg(ref.U.shift_fg(m3, dx=3, dy=-2), scale_factor=1.2)
-    nb = m.astype(np.float64) / 255
-    want = (f.astype(np.float64) * nb + bg.astype(np.float64) * (1 - nb)).astype(np.uint8)
-    d = np.abs(R.replace_frame(fg, m3, bg, 3, -2, 1.2).astype(int) - want.astype(int))
-    assert d.max() <= 2 and (d > 0).mean() <= 1e-3
+        check(f"rescale_{sc}", R.rescale_fg(fg, sc), lambda: ref.U.rescale_fg(fg, scale_factor=sc), ties(1, 1e-4))
+
+    def want():   # replace.py:69-76 restated with the reference's own functions
+        f = ref.U.rescale_fg(ref.U.shift_fg(fg, dx=3, dy=-2), scale_factor=1.2)
+        m = ref.U.rescale_fg(ref.U.shift_fg(m3, dx=3, dy=-2), scale_factor=1.2)
+        nb = m.astype(np.float64) / 255
+        return (f.astype(np.float64) * nb + bg.astype(np.float64) * (1 - nb)).astype(np.uint8)
+    check("replace_frame", R.replace_frame(fg, m3, bg, 3, -2, 1.2), want, ties(2, 1e-3))
 
 
 @pytest.mark.parametrize("h,w,L", [(108, 192, 96), (216, 384, 96), (150, 110, 60), (96, 160, 160)])
-def test_color_correct(ref, h, w, L):
+def test_color_correct(ref, check, h, w, L):
     """color_correct (imgprocess.py:263-300) against the live reference: bit-exact (the float32 sequence is restated
     operation by operation; only the loop's mean is accumulated differently, see the oracle's docstring)."""
     from video_unscreen_b200 import synth
@@ -128,36 +195,36 @@ def test_color_correct(ref, h, w, L):
         alpha = np.minimum(alpha, segs[i])
         for col in ((60, 200, 40), (200, 30, 30)):
             c = np.array(col, np.uint8)
-            want = ref.U.color_correct(frames[i].copy(), alpha.copy(), c.copy(), target_long_side=L)
-            got = R.color_correct(frames[i], alpha, c, target_long_side=L)
-            assert np.array_equal(got, want), (i, col, int((got != want).sum()))
+            check(f"color_correct_{h}_{w}_{L}_{i}_{col[0]}", R.color_correct(frames[i], alpha, c, target_long_side=L),
+                  lambda: ref.U.color_correct(frames[i].copy(), alpha.copy(), c.copy(), target_long_side=L))
 
 
 @pytest.mark.parametrize("h,w,L,kind", [(120, 200, 100, 0), (216, 384, 192, 1), (270, 480, 540, 2), (200, 130, 90, 1)])
-def test_background_agent(h, w, L, kind):
+def test_background_agent(ref, check, h, w, L, kind):
     """BackgroundAgent.forward 'pcov' (bit-exact) and 'mean' (<= 2 LSB: cv2's HSV2BGR tail) against the live reference"""
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    from make_golden import bgmodel_case, load_reference
-    BA = load_reference(REF_ROOT)[3]
+    from make_golden import bgmodel_case
     img, m = bgmodel_case(h, w, h * 7 + kind, kind)
-    ag = BA(input_long_side=L)
-    assert np.array_equal(R.background_forward(img, m, "pcov", input_long_side=L), ag.forward(img.copy(), m.copy(), "pcov"))
-    d = np.abs(R.background_forward(img, m, "mean", input_long_side=L).astype(int) - ag.forward(img.copy(), m.copy(), "mean").astype(int))
-    assert d.max() <= 2      # where: the hole pixels of the scalar-tail columns (image width mod the SIMD width)
-    d = np.abs(R.background_forward(img, m, "rf", input_long_side=L).astype(int) - ag.forward(img.copy(), m.copy(), "rf").astype(int))
-    assert d.max() <= 2      # the same HSV2BGR tail; the region fill itself agrees to 1e-9:
-    import unscreen.utils.region_fill as ref_rf
+    ag = ref.BA(input_long_side=L) if ref else None
+    key = f"bg_{h}_{w}_{L}_{kind}"
+    check(key + "_pcov", R.background_forward(img, m, "pcov", input_long_side=L), lambda: ag.forward(img.copy(), m.copy(), "pcov"))
+    # where: the hole pixels of the scalar-tail columns (image width mod the SIMD width)
+    check(key + "_mean", R.background_forward(img, m, "mean", input_long_side=L), lambda: ag.forward(img.copy(), m.copy(), "mean"), within(2))
+    # the same HSV2BGR tail; the region fill itself agrees to 1e-9:
+    check(key + "_rf", R.background_forward(img, m, "rf", input_long_side=L), lambda: ag.forward(img.copy(), m.copy(), "rf"), within(2))
     for f in (1.0, 0.5):
-        assert np.abs(R.regionfill(img[:, :, 1], m > 0, f) - ref_rf.regionfill(img[:, :, 1].copy(), m > 0, f)).max() <= 1e-9
-    ag2 = BA(input_long_side=L, dilation_ksize=3, dilation_iters=2, pcov_ksize=3)
-    want = ag2.forward(img.copy(), m.copy(), "pcov")
-    assert np.array_equal(R.background_forward(img, m, "pcov", input_long_side=L, dilation_ksize=3, dilation_iters=2, pcov_ksize=3), want)
+        def want():
+            import unscreen.utils.region_fill as ref_rf
+            return ref_rf.regionfill(img[:, :, 1].copy(), m > 0, f)
+        check(f"{key}_regionfill_{f}", R.regionfill(img[:, :, 1], m > 0, f), want, within(1e-9))
+    ag2 = ref.BA(input_long_side=L, dilation_ksize=3, dilation_iters=2, pcov_ksize=3) if ref else None
+    check(key + "_pcov_k3", R.background_forward(img, m, "pcov", input_long_side=L, dilation_ksize=3, dilation_iters=2, pcov_ksize=3),
+          lambda: ag2.forward(img.copy(), m.copy(), "pcov"))
 
 
 def test_contour_model_vs_cv2():
     """every contour of cv2.findContours(RETR_LIST): its drawContours(FILLED) paint and its contourArea, against the
-    closed-form model, as multisets, on random small shapes (dense, sparse, closed)"""
-    import cv2
+    closed-form model, as multisets, on random small shapes (dense, sparse, closed); needs cv2, not the reference"""
+    cv2 = pytest.importorskip("cv2")
     rng = np.random.default_rng(5)
     for trial in range(400):
         h, w = rng.integers(3, 16, 2)
@@ -170,11 +237,10 @@ def test_contour_model_vs_cv2():
 
 
 @pytest.mark.parametrize("seed", range(8))
-def test_remove_invalid_objects(ref, seed):
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+def test_remove_invalid_objects(ref, check, seed):
     from make_golden import OBJ_CFGS, objects_case
     h, w = [(100, 160), (160, 100), (90, 90), (120, 210)][seed % 4]
     a, seg = objects_case(h, w, 900 + seed)
-    for cfg in OBJ_CFGS:
-        assert np.array_equal(R.remove_invalid_objects(cfg, a), ref.U.remove_invalid_objects(cfg, a.copy()))
-        assert np.array_equal(R.remove_invalid_objects(cfg, a, seg), ref.U.remove_invalid_objects(cfg, a.copy(), seg.copy()))
+    for j, cfg in enumerate(OBJ_CFGS):
+        check(f"objects_{seed}_{j}", R.remove_invalid_objects(cfg, a), lambda: ref.U.remove_invalid_objects(cfg, a.copy()))
+        check(f"objects_{seed}_{j}_seg", R.remove_invalid_objects(cfg, a, seg), lambda: ref.U.remove_invalid_objects(cfg, a.copy(), seg.copy()))
