@@ -358,8 +358,8 @@ int vu_pcov_round(const uint8_t* img_in, const uint8_t* valid_in, int in_pitch_p
  * filled polygon scores saliency = sum(score_map under it) / (h w) and consensus = mean(segmask under it) / 255 with
  * (saliency > saliency_thr && consensus > consensus_thr) || saliency > 10 saliency_thr.  alpha, segmask, out: [n][h][w]
  * (segmask = alpha for the one-argument form of the reference); score_map: [h][w] float64 (get_score_map, :155-178), shared by
- * the frames.  status[i] = number of contours of frame i; a frame with more than max_objects contours (or nested deeper
- * than 65 levels) has status[i] > max_objects and an undefined output: call again with a larger workspace.  Everything
+ * the frames.  status[i] = number of contours of frame i; a frame with more than max_objects contours has
+ * status[i] > max_objects and an undefined output: call again with a larger workspace.  Nesting may be of any depth.  Everything
  * stays on the device.  workspace: vu_remove_objects_workspace_bytes(n, h, w, max_objects), 16-byte aligned. */
 size_t vu_remove_objects_workspace_bytes(int n, int h, int w, int max_objects);
 int vu_remove_invalid_objects(const uint8_t* alpha, const uint8_t* segmask, const double* score_map, int n, int h, int w,

@@ -692,8 +692,161 @@ def contour_objects(X):
     return objs
 
 
-def remove_invalid_objects(cfg, alpha, segmask=None):
-    """unscreen/utils/maskprocess.py:77-152 on the closed-form contour model above (does not mutate ``alpha``)."""
+def contour_records(X, segmask, score_map):
+    """The closed form of ``contour_objects`` in whole-array operations: one labelling per class instead of one per
+    contour (remove_invalid_objects_fast, one x86 core: 0.3 s for a blobby 1080p matte with 1 500 contours, 3.7 s for a
+    4K noise matte with 350 000).  X: bool [h,w]; segmask uint8 [h,w]; score_map
+    float64 [h,w].  Returns (records, lab, parent, nf):
+
+      records: dict of per-contour arrays, one entry per contour (every label but the outside), in label order:
+        ``label``, ``hole`` (bool), ``depth`` (components odd, holes even), ``parent`` (label), ``area`` (cv2.contourArea),
+        ``count`` / ``segsum`` / ``score``: pixels, mask sum and score-map sum under the FILLED contour;
+      lab: int32 [h+2, w+2] label image of the frame padded by one background pixel: 1..nf foreground (8-connected),
+        nf+1.. background (4-connected), lab[0, 0] = the outside;
+      parent: the nesting tree over labels (the outside is its own parent).
+
+    Every sum but ``score`` is an integer and exact; ``score`` is summed in another order than ``contour_objects`` (and
+    the device), so it agrees with them to rounding only."""
+    from scipy import ndimage as ndi
+    X = np.asarray(X, bool)
+    h, w = X.shape
+    P = np.pad(X, 1)
+    fl, nf = ndi.label(P, np.ones((3, 3), int))
+    bl, _ = ndi.label(~P, np.array([[0, 1, 0], [1, 1, 1], [0, 1, 0]]))
+    lab = np.where(P, fl, bl + nf).astype(np.int32)
+    flat = lab.ravel()
+    outer = int(flat[0])
+    n = int(flat.max()) + 1                                  # label 0 is unused
+    # the parent of a set = the set of the pixel left of its first pixel in raster order
+    labels, first = np.unique(flat, return_index=True)
+    parent = np.zeros(n, np.int64)
+    parent[labels] = flat[first - 1]
+    parent[outer] = outer
+    # depths by pointer jumping
+    depth = (parent != np.arange(n)).astype(np.int64)
+    anc = parent.copy()
+    while np.any(depth[anc]):
+        depth, anc = depth + depth[anc], anc[anc]
+    # per-set sums over the frame
+    inner = lab[1:-1, 1:-1].ravel()
+    cnt = np.bincount(inner, minlength=n).astype(np.int64)
+    seg = np.bincount(inner, weights=np.asarray(segmask, np.float64).ravel(), minlength=n).astype(np.int64)
+    score = np.bincount(inner, weights=np.asarray(score_map, np.float64).ravel(), minlength=n)
+    # the ring of a hole: the pixels of its parent component 4-adjacent to it, each counted once per hole
+    fgpix = X.ravel()
+    lf = inner[fgpix]
+    pf = parent[lf]
+    nbs = [lab[1:-1, :-2], lab[1:-1, 2:], lab[:-2, 1:-1], lab[2:, 1:-1]]
+    nbs = [b.ravel()[fgpix] for b in nbs]
+    sg_f = np.asarray(segmask, np.float64).ravel()[fgpix]
+    sc_f = np.asarray(score_map, np.float64).ravel()[fgpix]
+    rcnt, rseg, rscore = np.zeros(n, np.int64), np.zeros(n, np.int64), np.zeros(n)
+    for j, b in enumerate(nbs):
+        m = (b > nf) & (b != pf)
+        for q in range(j):
+            m &= b != nbs[q]
+        rcnt += np.bincount(b[m], minlength=n)
+        rseg += np.bincount(b[m], weights=sg_f[m], minlength=n).astype(np.int64)
+        rscore += np.bincount(b[m], weights=sc_f[m], minlength=n)
+    del nbs, lf, pf
+    # L: pixel edges between a component and its parent (its outer border) or one of its holes (that hole's border)
+    L = np.zeros(n, np.int64)
+    for la, lb in ((lab[:, :-1], lab[:, 1:]), (lab[:-1, :], lab[1:, :])):
+        fa, fb = la <= nf, lb <= nf
+        e = fa != fb
+        lfg = np.where(fa, la, lb)[e]
+        lbg = np.where(fa, lb, la)[e]
+        L += np.bincount(np.where(lbg == parent[lfg], lfg, lbg), minlength=n)
+    # 2x2 windows with one foreground pixel and three pixels of one background set: n1 of the component when that set is
+    # its parent, else n3 of that hole
+    win = (lab[:-1, :-1], lab[:-1, 1:], lab[1:, :-1], lab[1:, 1:])
+    nfg = sum((x <= nf).astype(np.int8) for x in win)
+    one = nfg == 1
+    ws = [x[one] for x in win]
+    lfg = np.max([np.where(x <= nf, x, 0) for x in ws], axis=0)
+    bmin = np.min([np.where(x <= nf, n, x) for x in ws], axis=0)
+    bmax = np.max([np.where(x <= nf, 0, x) for x in ws], axis=0)
+    same = bmin == bmax
+    lfg, b = lfg[same], bmin[same]
+    nw = np.bincount(np.where(b == parent[lfg], lfg, b), minlength=n)
+    del win, nfg, one, ws
+    # subtree totals, deepest level first: a filled contour covers its set and everything nested in it
+    order = np.argsort(depth, kind="stable")[::-1]
+    ds = depth[order]
+    bounds = np.flatnonzero(np.diff(ds)) + 1
+    for grp in np.split(order, bounds):
+        if depth[grp[0]] == 0:
+            continue
+        p = parent[grp]
+        np.add.at(cnt, p, cnt[grp])
+        np.add.at(seg, p, seg[grp])
+        np.add.at(score, p, score[grp])
+    ids = np.delete(np.arange(1, n), outer - 1)
+    hole = ids > nf
+    B = (L[ids] - nw[ids]) / 2.0
+    rec = {
+        "label": ids, "hole": hole, "depth": depth[ids], "parent": parent[ids],
+        "area": np.where(hole, cnt[ids] + B - 1, cnt[ids] - B - 1),
+        "count": cnt[ids] + np.where(hole, rcnt[ids], 0),
+        "segsum": seg[ids] + np.where(hole, rseg[ids], 0),
+        "score": score[ids] + np.where(hole, rscore[ids], 0.0),
+    }
+    return rec, lab, parent, nf
+
+
+def remove_invalid_objects_fast(cfg, alpha, segmask=None, return_records=False):
+    """``remove_invalid_objects`` on ``contour_records``: the same result (tests/test_oracle_objects_fast.py), fast
+    enough for 1080p and 4K frames.  With ``return_records`` also the records, plus per contour ``saliency``,
+    ``consensus``, ``valid`` and the decision margins: ``sal_margin`` = relative distance of the saliency from
+    saliency_thr and from 10 * saliency_thr (the nearer one), ``con_margin`` = relative distance of the consensus from
+    consensus_thr.  Only the saliency is a floating-point sum whose order matters (the consensus is an integer sum
+    divided the same way everywhere), so ``sal_margin`` of the contours with area >= 100 bounds what summation order
+    could flip."""
+    saliency_thr = cfg['objectremoval']['saliency_thr']
+    consensus_thr = cfg['objectremoval']['consensus_thr']
+    if segmask is None:
+        segmask = alpha
+    h, w = alpha.shape
+    rec, lab, parent, nf = contour_records(alpha > 0, segmask, build_score_map(h, w, cfg))
+    saliency = rec["score"] / float(h * w)
+    consensus = rec["segsum"] / rec["count"] / 255.
+    valid = ~(rec["area"] < 100) & (((saliency > saliency_thr) & (consensus > consensus_thr)) | (saliency > saliency_thr * 10))
+    # painted: the pixel's set or one of its ancestors is a valid contour (pointer jumping up the tree) ...
+    n = parent.size
+    flag = np.zeros(n, bool)
+    flag[rec["label"]] = valid
+    anc = parent.copy()
+    while True:
+        flag = flag | flag[anc]
+        nxt = anc[anc]
+        if np.array_equal(nxt, anc):
+            break
+        anc = nxt
+    vhole = np.zeros(n, bool)
+    vhole[rec["label"][rec["hole"] & valid]] = True
+    keep = flag[lab[1:-1, 1:-1]]
+    # ... or it is on the ring of a valid hole
+    for b in (lab[1:-1, :-2], lab[1:-1, 2:], lab[:-2, 1:-1], lab[2:, 1:-1]):
+        keep |= vhole[b]
+    out = np.where(keep & (alpha > 0), alpha, 0).astype(alpha.dtype)
+    if not return_records:
+        return out
+    rec.update(saliency=saliency, consensus=consensus, valid=valid,
+               sal_margin=np.minimum(np.abs(saliency - saliency_thr) / saliency_thr,
+                                     np.abs(saliency - 10 * saliency_thr) / (10 * saliency_thr)),
+               con_margin=np.abs(consensus - consensus_thr) / consensus_thr)
+    return out, rec
+
+
+def decision_margin(rec):
+    """the smallest ``sal_margin`` over the contours whose scores decide anything (area >= 100); inf without any"""
+    m = rec["sal_margin"][~(rec["area"] < 100)]
+    return float(m.min()) if m.size else float("inf")
+
+
+def remove_invalid_objects(cfg, alpha, segmask=None, objs=None):
+    """unscreen/utils/maskprocess.py:77-152 on the closed-form contour model above (does not mutate ``alpha``).
+    ``objs``: contour_objects(alpha > 0) when the caller already has it."""
     saliency_thr = cfg['objectremoval']['saliency_thr']
     consensus_thr = cfg['objectremoval']['consensus_thr']
     if segmask is None:
@@ -701,7 +854,7 @@ def remove_invalid_objects(cfg, alpha, segmask=None):
     h, w = alpha.shape
     score_map = build_score_map(h, w, cfg)
     valid = np.zeros((h, w), bool)
-    for fill, area in contour_objects(alpha > 0):
+    for fill, area in (contour_objects(alpha > 0) if objs is None else objs):
         if area < 100:
             continue
         saliency = score_map[fill].sum() / float(h * w)

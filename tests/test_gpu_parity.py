@@ -824,22 +824,8 @@ def test_remove_invalid_objects_shapes(vu):
     import os, sys
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
     from make_golden import OBJ_CFGS
-    h, w = 96, 128
-    a = np.zeros((h, w), np.uint8)
-    a[10:70, 10:90] = 200
-    a[20:60, 20:80] = 0            # hole
-    a[30:50, 30:60] = 150          # island in the hole
-    a[35:45, 38:52] = 0            # its own hole
-    a[38:42, 42:48] = 90           # island in that
-    a[0:12, 100:128] = 255         # touches the border: area (11 * 27) > 100
-    a[80:90, 5:15] = 77            # 10 x 10: contour area 81 < 100
-    a[80:91, 30:41] = 77           # 11 x 11: contour area 100
-    for k in range(15):            # diagonal chain: 8-connected, area 0
-        a[75 + k, 60 + k] = 255
-    a[70, 95] = 255                # diagonal contact with the big ring's corner pixel (69, 89)?  no: isolated pixel
-    a[70, 90] = 255                # this one touches (69, 89) diagonally: joins the ring
-    seg = np.zeros((h, w), np.uint8)
-    seg[:, :70] = 255
+    from test_oracle_objects_fast import handmade_objects
+    a, seg = handmade_objects()
     for cfg in OBJ_CFGS:
         for s in (None, seg):
             assert np.array_equal(vu.U.remove_invalid_objects(cfg, a, s), R.remove_invalid_objects(cfg, a, s)), (cfg, s is None)

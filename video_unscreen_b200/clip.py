@@ -283,12 +283,15 @@ def color_correct_clip(frames, alpha, bg_color, target_long_side=960, mean_exp=0
 
 
 def green_clip(frames, segmasks, cf_agent, trimap_agent, chunk=24, bg_color=None, bg_tile=None, color_correct=False, streams=2, fused=True, out=None,
-               remove_objects=None, max_objects=16384):
+               remove_objects=None, max_objects=16384, tracked=None):
     """the green-screen loop of tools/unscreen/green.py:70-138 without its CNN
     stages (alpha := colour-filter alpha): cf predict -> [remove_invalid_objects, green.py:106-109, when
-    ``remove_objects`` = the script's cfg dict is given: the matte the trimap and get_fg see is the cleaned one; every
-    frame is scored against its segmentation mask, like the frames after the first in the script] -> trimap with bg
-    colour -> [color_correct, green.py:120, when asked for] -> bgimg[alpha<128] = frame[...] -> get_fg.  Everything
+    ``remove_objects`` = the script's cfg dict is given: the matte the trimap and get_fg see is the cleaned one] -> trimap
+    with bg colour -> [color_correct, green.py:120, when asked for] -> bgimg[alpha<128] = frame[...] -> get_fg.
+    Like the script, an untracked frame is scored against its segmentation mask (remove_invalid_objects(cfg, alpha,
+    segmask)) and a tracked one against its own colour-filter alpha (remove_invalid_objects(cfg, alpha)): ``tracked``
+    = per-frame booleans (list, ndarray or device tensor of length n; a device tensor when the call is captured into a
+    CUDA graph), None = no frame tracked.  Everything
     stays on the device; a frame with more than ``max_objects`` contours raises after the clip (one read-back).
     Returns alpha, trimap, fg, bg.
     ``bg_color`` ((3,) BGR, host) / ``bg_tile`` ([1,4,3] device) default to the agent's background colour; pass them
@@ -312,11 +315,16 @@ def green_clip(frames, segmasks, cf_agent, trimap_agent, chunk=24, bg_color=None
         from .unscreen.utils.maskprocess import _score_map_dev
         score_map = _score_map_dev(h, w, remove_objects, dev)
         sal_thr, con_thr = remove_objects['objectremoval']['saliency_thr'], remove_objects['objectremoval']['consensus_thr']
+        if tracked is not None:
+            tracked = torch.as_tensor(np.asarray(tracked, bool) if not torch.is_tensor(tracked) else tracked, device=dev).bool()
+            if tracked.shape != (n,):
+                raise ValueError(f"tracked must hold one boolean per frame ({n}), got shape {tuple(tracked.shape)}")
     def body(s, e):
         # every stage writes straight into its slice of the clip-sized results
         if remove_objects is not None:
             a = cf_predict_clip(frames[s:e], segmasks[s:e], cf_agent, chunk=chunk)
-            a, st = ops.remove_invalid_objects(a, segmasks[s:e], score_map, sal_thr, con_thr, max_objects, out=alpha[s:e])
+            sm = segmasks[s:e] if tracked is None else torch.where(tracked[s:e, None, None], a, segmasks[s:e])
+            a, st = ops.remove_invalid_objects(a, sm, score_map, sal_thr, con_thr, max_objects, out=alpha[s:e])
             statuses.append(st)
             trimap_clip(a, trimap_agent, frames[s:e], bg_color, chunk=chunk, out=tri[s:e])
             if color_correct:

@@ -283,28 +283,22 @@ __global__ void __launch_bounds__(1024) obj_tree_kernel(int h, int w, void* wsba
   if (*ws.overflow) return;
   const int nr = *ws.nroots;
   // kind: foreground roots have a foreground pixel: a component's depth is odd (children of the outside), a hole's even
-  // depth by relaxation: parent ids are smaller than child ids, a handful of sweeps settle it
+  // depth by relaxation, one level per sweep: sweep s gives depth s + 2 to the children of the nodes of depth s + 1 (a
+  // node written in this sweep is not read as a parent in it, so the sweep is race-free).  The tree has nr nodes, so it
+  // is at most nr deep and the sweeps stop, at the latest, after nr of them
   for (int k = threadIdx.x; k < nr; k += blockDim.x) ws.depth[k] = ws.up[k] < 0 ? 1 : 0;
   __syncthreads();
   int maxd = 1;
-  for (int sweep = 0; sweep < 64; ++sweep) {
+  for (int sweep = 0; sweep < nr; ++sweep) {
     int changed = 0;
     for (int k = threadIdx.x; k < nr; k += blockDim.x) {
       if (ws.depth[k] == 0) {
         const int dp = ws.depth[ws.up[k]];
-        if (dp > 0 && dp == sweep + 1) { ws.depth[k] = dp + 1; changed = 1; }
+        if (dp == sweep + 1) { ws.depth[k] = dp + 1; changed = 1; }
       }
     }
     if (!__syncthreads_or(changed)) break;
     maxd = sweep + 2;
-  }
-  {   // deeper than 65 levels of nesting: give up on the frame (reported like too many contours)
-    int bad = 0;
-    for (int k = threadIdx.x; k < nr; k += blockDim.x) bad |= ws.depth[k] == 0;
-    if (__syncthreads_or(bad)) {
-      if (threadIdx.x == 0) { *ws.overflow = 1; *ws.nroots = 0x7fffffff; }
-      return;
-    }
   }
   // subtree totals, deepest level first (only the sums a filled contour needs: pixels, mask sum, saliency sum)
   for (int d = maxd; d >= 2; --d) {
@@ -403,12 +397,13 @@ extern "C" int vu_remove_invalid_objects(const uint8_t* alpha, const uint8_t* se
   obj_stats_kernel<<<dim3(gx, n), OT, 0, st>>>(alpha, segmask, score_map, h, w, workspace, max_objects);
   obj_tree_kernel<<<n, 1024, 0, st>>>(h, w, workspace, max_objects, saliency_thr, consensus_thr);
   obj_apply_kernel<<<dim3(gx, n), OT, 0, st>>>(alpha, h, w, workspace, max_objects, out);
-  // status[i] = number of contours of frame i, or -1 when it had more than max_objects (its output is then undefined)
+  // status[i] = number of contours of frame i; more than max_objects: the frame's output is undefined (the caller redoes
+  // it with a larger table)
   for (int i = 0; i < n; ++i) {
     const ObjWs ws = ws_of(workspace, i, npix, max_objects);
     int e = record_cuda(cudaMemcpyAsync(status + i, ws.nroots, sizeof(int), cudaMemcpyDeviceToDevice, st));
     if (e) return e;
   }
-  note_launch(6);
+  note_launch(7);
   VU_RETURN_LAUNCH();
 }

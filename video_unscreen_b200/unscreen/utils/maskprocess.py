@@ -95,7 +95,5 @@ def remove_invalid_objects(cfg, alpha, segmask=None, saliency_thr=0.001, consens
         worst = int(status.max().item())
         if worst <= max_objects:
             break
-        if worst > h * w + 1:          # nested deeper than the tree kernel handles
-            raise RuntimeError("remove_invalid_objects: objects nested deeper than 65 levels")
         max_objects = worst
     return back(out, as_np)
