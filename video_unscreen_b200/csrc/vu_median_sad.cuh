@@ -24,7 +24,8 @@
 //            stage B over 0..255 (12 probes).  Always exact; only the speed
 //            depends on the data.
 //
-// Layout.  A warp owns SEG = 128/SPLIT consecutive bytes of every frame.  The
+// Layout of the direct kernel (the TMA tile kernel below has its own, and the
+// search is written for both).  A warp owns SEG = 128/SPLIT consecutive bytes of every frame.  The
 // frames are dealt to SPLIT lane groups ("parts"): part p holds frames
 // f = SPLIT*i + p.  Lane l of a part holds its 4 bytes of all those frames: one
 // coalesced LDG.32 per frame, every load of the warp in flight at once.  Slot
@@ -91,28 +92,41 @@ __device__ __forceinline__ void static_for(F&& f) {
 constexpr unsigned BIG = 0x7fffffffu;
 constexpr unsigned FULL = 0xffffffffu;
 
-// S(m[j]) over all frames of the warp's segment for the 4 elements of the lane.
+// The search below is written for any register layout of this form: a lane holds E elements, register d[E*k + j]
+// holds 4 frames of element j (k = 0..K-1), and the frames of one element are spread over the lanes that differ
+// only in the lane bits XMASK (a contiguous run of bits, or 0 when one lane holds all frames of its elements).
+__host__ __device__ constexpr int lowest_bit(unsigned x) { return x & 1u ? 0 : 1 + lowest_bit(x >> 1); }
+template <unsigned XMASK>
+__host__ __device__ constexpr int parts_of() { return XMASK ? (int)(XMASK >> lowest_bit(XMASK)) + 1 : 1; }   // lanes that share an element
+
+// S(m[j]) over all frames of the warp's segment for the E elements of the lane.
 // RANGE: probes outside 0..255 are allowed and evaluate to BIG.
-template <int SPLIT, int G, bool RANGE>
-__device__ __forceinline__ void eval_s(const unsigned (&d)[4 * G], const int (&m)[4], int delta, unsigned (&S)[4]) {
-  constexpr int LPS = 32 / SPLIT;
-  unsigned q[4], s[4];
+template <int E, unsigned XMASK, int K, bool RANGE>
+__device__ __forceinline__ void eval_s(const unsigned (&d)[E * K], const int (&m)[E], int delta, unsigned (&S)[E]) {
+  constexpr int NA = E < 4 ? 4 / E : 1;   // accumulators per element: at least 4 independent VABSDIFF4 chains per lane
+  static_assert(K % NA == 0, "words per element must split evenly over the accumulators");
+  unsigned q[E], s[E][NA];
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
+  for (int j = 0; j < E; ++j) {
     q[j] = (unsigned)(RANGE ? min(max(m[j], 0), 255) : m[j]) * 0x01010101u;
-    s[j] = 0;
+#pragma unroll
+    for (int a = 0; a < NA; ++a) s[j][a] = 0;
   }
 #pragma unroll
-  for (int g = 0; g < G; ++g) {
+  for (int k = 0; k < K; ++k) {
 #pragma unroll
-    for (int j = 0; j < 4; ++j) s[j] = sad_acc(d[4 * g + j], q[j], s[j]);
+    for (int j = 0; j < E; ++j) s[j][k % NA] = sad_acc(d[E * k + j], q[j], s[j][k % NA]);
   }
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
+  for (int j = 0; j < E; ++j) {
+    unsigned t = s[j][0];
 #pragma unroll
-    for (int o = LPS; o < 32; o <<= 1) s[j] += __shfl_xor_sync(FULL, s[j], o);
-    s[j] += (unsigned)(delta * m[j]);
-    S[j] = (RANGE && (m[j] < 0 || m[j] > 255)) ? BIG : s[j];
+    for (int a = 1; a < NA; ++a) t += s[j][a];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1)
+      if (XMASK & o) t += __shfl_xor_sync(FULL, t, o);
+    t += (unsigned)(delta * m[j]);
+    S[j] = (RANGE && (m[j] < 0 || m[j] > 255)) ? BIG : t;
   }
 }
 
@@ -120,27 +134,27 @@ __device__ __forceinline__ void eval_s(const unsigned (&d)[4 * G], const int (&m
 // (a, a+F(K0)).  On return r is the minimiser among them, smin = S(r), and
 // sl / sr are S(r-1) / S(r+1), or BIG where that neighbour is the bracket's
 // original end (never evaluated).  2 + (K0 - 4) evaluations of S.
-template <int SPLIT, int G, bool RANGE>
-__device__ __forceinline__ void fib_search(const unsigned (&d)[4 * G], int delta, int k0, int fa, int fb, int fc, int (&a)[4], int (&r)[4],
-                                           unsigned (&smin)[4], unsigned (&sl)[4], unsigned (&sr)[4]) {
-  unsigned S1[4], S2[4];
+template <int E, unsigned XMASK, int K, bool RANGE>
+__device__ __forceinline__ void fib_search(const unsigned (&d)[E * K], int delta, int k0, int fa, int fb, int fc, int (&a)[E], int (&r)[E],
+                                           unsigned (&smin)[E], unsigned (&sl)[E], unsigned (&sr)[E]) {
+  unsigned S1[E], S2[E];
   {
-    int i1[4], i2[4];
+    int i1[E], i2[E];
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < E; ++j) {
       i1[j] = a[j] + fb;
       i2[j] = a[j] + fa;
       sl[j] = sr[j] = BIG;
     }
-    eval_s<SPLIT, G, RANGE>(d, i1, delta, S1);
-    eval_s<SPLIT, G, RANGE>(d, i2, delta, S2);
+    eval_s<E, XMASK, K, RANGE>(d, i1, delta, S1);
+    eval_s<E, XMASK, K, RANGE>(d, i2, delta, S2);
   }
 #pragma unroll 1
   for (int k = k0; k >= 5; --k) {
-    int nidx[4];
-    bool left[4];
+    int nidx[E];
+    bool left[E];
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < E; ++j) {
       left[j] = S1[j] <= S2[j];
       if (left[j]) {
         sr[j] = S2[j];
@@ -153,10 +167,10 @@ __device__ __forceinline__ void fib_search(const unsigned (&d)[4 * G], int delta
         nidx[j] = a[j] + fb;
       }
     }
-    unsigned Sn[4];
-    eval_s<SPLIT, G, RANGE>(d, nidx, delta, Sn);
+    unsigned Sn[E];
+    eval_s<E, XMASK, K, RANGE>(d, nidx, delta, Sn);
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < E; ++j) {
       if (left[j]) S1[j] = Sn[j];
       else S2[j] = Sn[j];
     }
@@ -167,7 +181,7 @@ __device__ __forceinline__ void fib_search(const unsigned (&d)[4 * G], int delta
   }
   // k == 4: bracket (a, a+3), S1 = S(a+1), S2 = S(a+2)
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
+  for (int j = 0; j < E; ++j) {
     if (S1[j] <= S2[j]) {
       r[j] = a[j] + 1;
       smin[j] = S1[j];
@@ -180,25 +194,37 @@ __device__ __forceinline__ void fib_search(const unsigned (&d)[4 * G], int delta
   }
 }
 
-// SS = stride of the 4 sample groups of stage A (0: no stage A, straight to the full search)
-template <int SPLIT, int G, int SS>
-__device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n, int delta) {
-  int a[4], r[4];
-  unsigned smin[4], sl[4], sr[4];
+template <int E>
+__device__ __forceinline__ bool open_any(const int (&L)[E], const int (&R)[E]) {
+  bool o = false;
+#pragma unroll
+  for (int j = 0; j < E; ++j) o |= L[j] < R[j];
+  return o;
+}
+
+// SS = stride of the 4 sample words of stage A (0: no stage A, straight to the full search).
+// Returns the median of element j in byte j.
+template <int E, unsigned XMASK, int K, int SS>
+__device__ __forceinline__ unsigned sad_median(const unsigned (&d)[E * K], int n, int delta) {
+  int a[E], r[E];
+  unsigned smin[E], sl[E], sr[E];
   bool full = (SS == 0);
   if (SS > 0) {
-    // ---- stage A: every part estimates 4/SPLIT of the lane's elements as the lower median of 16 of ITS frames
-    // (bisection on the slope of S), then the parts swap their estimates ----
-    constexpr int EPP = 4 / SPLIT;   // elements per part
-    const int part = (threadIdx.x & 31) / (32 / SPLIT);
+    // ---- stage A: every part (one of the lanes that share an element) estimates E/PARTS of the lane's elements as
+    // the lower median of 16 of ITS frames (bisection on the slope of S), then the parts swap their estimates ----
+    constexpr int PARTS = parts_of<XMASK>();
+    constexpr int PSHIFT = XMASK ? lowest_bit(XMASK) : 0;
+    constexpr int EPP = E / PARTS;   // elements per part
+    const int lane = threadIdx.x & 31;
+    const int part = (lane & XMASK) >> PSHIFT;
     unsigned smp[EPP][4];
 #pragma unroll
     for (int e = 0; e < EPP; ++e)
 #pragma unroll
       for (int t = 0; t < 4; ++t) {
-        unsigned v = d[4 * (t * SS) + e];
+        unsigned v = d[E * (t * SS) + e];
 #pragma unroll
-        for (int p = 1; p < SPLIT; ++p) v = (part == p) ? d[4 * (t * SS) + p * EPP + e] : v;
+        for (int p = 1; p < PARTS; ++p) v = (part == p) ? d[E * (t * SS) + p * EPP + e] : v;
         smp[e][t] = v;
       }
     int est[EPP];
@@ -219,31 +245,31 @@ __device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n
       }
     }
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int c = __shfl_sync(FULL, est[j % EPP], (j / EPP) * (32 / SPLIT) + (threadIdx.x & (32 / SPLIT - 1)));
+    for (int j = 0; j < E; ++j) {
+      const int c = PARTS == 1 ? est[j] : __shfl_sync(FULL, est[j % EPP], (lane & ~XMASK) | ((j / EPP) << PSHIFT));
       a[j] = min(max(c - 10, -1), 235);   // interior a+1 .. a+20 within 0..255
     }
     // ---- stage B: the 20 values around the estimate ----
-    fib_search<SPLIT, G, false>(d, delta, 8, 13, 8, 5, a, r, smin, sl, sr);
+    fib_search<E, XMASK, K, false>(d, delta, 8, 13, 8, 5, a, r, smin, sl, sr);
     bool fail = false;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) fail |= (sl[j] == BIG && r[j] > 0) || (sr[j] == BIG && r[j] < 255);
+    for (int j = 0; j < E; ++j) fail |= (sl[j] == BIG && r[j] > 0) || (sr[j] == BIG && r[j] < 255);
     full = __any_sync(FULL, fail);
   }
   if (full) {
 #pragma unroll
-    for (int j = 0; j < 4; ++j) a[j] = -1;
-    fib_search<SPLIT, G, true>(d, delta, 14, 233, 144, 89, a, r, smin, sl, sr);   // interior -1+1 .. 375: covers 0..255
+    for (int j = 0; j < E; ++j) a[j] = -1;
+    fib_search<E, XMASK, K, true>(d, delta, 14, 233, 144, 89, a, r, smin, sl, sr);   // interior -1+1 .. 375: covers 0..255
   }
-  int lo[4], hi[4];
+  int lo[E], hi[E];
 #pragma unroll
-  for (int j = 0; j < 4; ++j) lo[j] = hi[j] = r[j];
+  for (int j = 0; j < E; ++j) lo[j] = hi[j] = r[j];
   if (!(n & 1)) {
     // even n: minimisers form the plateau [x_lo, x_hi]
-    bool openL[4], openR[4];
+    bool openL[E], openR[E];
     bool any = false;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < E; ++j) {
       openL[j] = openR[j] = false;
       if (sl[j] == smin[j]) { lo[j] = r[j] - 1; openL[j] = lo[j] > 0; }
       if (sr[j] == smin[j]) { hi[j] = r[j] + 1; openR[j] = hi[j] < 255; }
@@ -252,14 +278,14 @@ __device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n
     // walk the open ends, one probe per lane and round
 #pragma unroll 1
     for (int it = 0; it < 4 && __any_sync(FULL, any); ++it) {
-      int idx[4];
-      unsigned S[4];
+      int idx[E];
+      unsigned S[E];
 #pragma unroll
-      for (int j = 0; j < 4; ++j) idx[j] = openL[j] ? lo[j] - 1 : (openR[j] ? hi[j] + 1 : r[j]);
-      eval_s<SPLIT, G, false>(d, idx, delta, S);
+      for (int j = 0; j < E; ++j) idx[j] = openL[j] ? lo[j] - 1 : (openR[j] ? hi[j] + 1 : r[j]);
+      eval_s<E, XMASK, K, false>(d, idx, delta, S);
       any = false;
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
+      for (int j = 0; j < E; ++j) {
         if (openL[j]) {
           if (S[j] == smin[j]) { --lo[j]; openL[j] = lo[j] > 0; }
           else openL[j] = false;
@@ -272,17 +298,17 @@ __device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n
     }
     // long plateaus (e.g. two-valued data): binary search for the ends (S == smin is monotone on either side)
     if (__any_sync(FULL, any)) {
-      int L[4], R[4];
+      int L[E], R[E];
 #pragma unroll
-      for (int j = 0; j < 4; ++j) { R[j] = lo[j]; L[j] = openL[j] ? 0 : lo[j]; }
-      while (__any_sync(FULL, (L[0] < R[0]) | (L[1] < R[1]) | (L[2] < R[2]) | (L[3] < R[3]))) {
-        int idx[4];
-        unsigned S[4];
+      for (int j = 0; j < E; ++j) { R[j] = lo[j]; L[j] = openL[j] ? 0 : lo[j]; }
+      while (__any_sync(FULL, open_any(L, R))) {
+        int idx[E];
+        unsigned S[E];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) idx[j] = (L[j] + R[j]) >> 1;
-        eval_s<SPLIT, G, false>(d, idx, delta, S);
+        for (int j = 0; j < E; ++j) idx[j] = (L[j] + R[j]) >> 1;
+        eval_s<E, XMASK, K, false>(d, idx, delta, S);
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
+        for (int j = 0; j < E; ++j)
           if (L[j] < R[j]) {
             const int mid = (L[j] + R[j]) >> 1;
             if (S[j] == smin[j]) R[j] = mid;
@@ -290,15 +316,15 @@ __device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n
           }
       }
 #pragma unroll
-      for (int j = 0; j < 4; ++j) { lo[j] = R[j]; L[j] = hi[j]; R[j] = openR[j] ? 255 : hi[j]; }
-      while (__any_sync(FULL, (L[0] < R[0]) | (L[1] < R[1]) | (L[2] < R[2]) | (L[3] < R[3]))) {
-        int idx[4];
-        unsigned S[4];
+      for (int j = 0; j < E; ++j) { lo[j] = R[j]; L[j] = hi[j]; R[j] = openR[j] ? 255 : hi[j]; }
+      while (__any_sync(FULL, open_any(L, R))) {
+        int idx[E];
+        unsigned S[E];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) idx[j] = (L[j] + R[j] + 1) >> 1;
-        eval_s<SPLIT, G, false>(d, idx, delta, S);
+        for (int j = 0; j < E; ++j) idx[j] = (L[j] + R[j] + 1) >> 1;
+        eval_s<E, XMASK, K, false>(d, idx, delta, S);
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
+        for (int j = 0; j < E; ++j)
           if (L[j] < R[j]) {
             const int mid = (L[j] + R[j] + 1) >> 1;
             if (S[j] == smin[j]) L[j] = mid;
@@ -306,12 +332,12 @@ __device__ __forceinline__ unsigned sad_median(const unsigned (&d)[4 * G], int n
           }
       }
 #pragma unroll
-      for (int j = 0; j < 4; ++j) hi[j] = L[j];
+      for (int j = 0; j < E; ++j) hi[j] = L[j];
     }
   }
   unsigned res = 0;
 #pragma unroll
-  for (int j = 0; j < 4; ++j) res |= (unsigned)((lo[j] + hi[j]) >> 1) << (8 * j);
+  for (int j = 0; j < E; ++j) res |= (unsigned)((lo[j] + hi[j]) >> 1) << (8 * j);
   return res;
 }
 
@@ -364,7 +390,7 @@ __global__ void __launch_bounds__(128, CTAS) median_sad_kernel(const uint8_t* __
     }
   });
   transpose_groups<G>(d);
-  const unsigned res = sad_median<SPLIT, G, SS>(d, n, delta);
+  const unsigned res = sad_median<4, 32u - LPS, G, SS>(d, n, delta);
   if (part == 0) reinterpret_cast<unsigned*>(out + (long long)seg * SEG)[li] = res;
 }
 
@@ -374,41 +400,75 @@ __global__ void __launch_bounds__(128, CTAS) median_sad_kernel(const uint8_t* __
 // Measured on the B200 (tools/ldgsts_ubench.cu, fetch only): "one row per frame" streams at 2.8 TB/s when a warp
 // fetches 64-byte rows on its own, at 5.9 TB/s with 128-byte rows and at 7.2 TB/s with 512-byte rows: requests must
 // cover whole 128-byte lines, and the direct kernel above (64 bytes per frame and warp) cannot get there.  Here a CTA
-// of WARPS warps owns tiles of WARPS adjacent segments (8 warps, SPLIT 2: 512 bytes of every frame).  The clip is
-// described to the TMA unit as a 2-D tensor [n frames][m bytes], and SPLIT boxes of {TILE bytes x 4G frames}
-// (cp.async.bulk.tensor.2d, one elected thread, completion counted in bytes on an mbarrier) bring the tile into
-// shared memory as rows of TILE bytes: no address arithmetic and no load instructions in the warps.  Frames past the end of the clip are zero-filled by the unit: pads are all 0 here and leave S through
-// delta = -(number of pads).  The warps are only loosely coupled: a warp waits for the tile on the mbarrier, moves its
-// segment to registers and transposes, bumps a counter and goes searching; the warp that bumps it last knows the
-// buffer is free and launches the fetch of the next tile, which then lands while everybody searches.
+// of WARPS warps owns tiles of WARPS adjacent segments of 16*C bytes (8 warps, C = 4: 512 bytes of every frame).  The
+// clip is described to the TMA unit as a 3-D tensor [n frames][m/128 chunks][128 bytes], and boxes of {TILE bytes x
+// BOX_ROWS frames} (cp.async.bulk.tensor.3d with the 128-byte swizzle, one elected thread, completion counted in bytes
+// on an mbarrier) bring the tile into shared memory as rows of TILE bytes.  The swizzle works on 128-byte units: unit
+// R = f*COLS + col (frame f, 128-byte column col) keeps its 16-byte chunk c at chunk c ^ (R & 7).  (With one box per
+// 128-byte column the rows fetched were only 128 bytes long, and the fetch capped the kernel at ~4.5 TB/s.)  Frames past the end of the clip are zero-filled by the
+// unit: pads are all 0 here and leave S through delta = -(number of pads).  The warps are only loosely coupled: a
+// warp waits for the tile on the mbarrier, moves its segment to registers, bumps a counter and goes searching; the
+// warp that bumps it last knows the buffer is free and launches the fetch of the next tile, which then lands while
+// everybody searches.
+//
+// Layout.  ldmatrix.m16n16.trans.b8 reads a 16 x 16 byte block (16 row addresses, 16 bytes each) and hands lane l
+// two words: rows 4*(l&3) .. +3 of block columns l>>2 and (l>>2)+8, i.e. "4 rows of one column" - four frames of one
+// element when the rows are frames - with no byte transposes on the ALU pipe.  The rows of one block need not be
+// adjacent: rows 4q .. 4q+3 (the ones lane quad member q receives) are 4 frames of the warp's 16-byte column block
+// q % C.  So a lane holds E = 2 elements (columns i and i+8 of column block q % C, i = l>>2), and the frames of an
+// element are dealt to the P = 4/C quad members q, q+C, ..: with C = 4 one lane holds every frame of its two elements
+// and S needs no shuffle; with C = 2 two lanes hold half the frames each (shfl_xor 2).  Word k = 2j+M (matrix M of the
+// j-th ldmatrix.x2) of quad member q holds frames 8Pj + 8(q/C) + 4((M^q)&1) + 0..3.  Banks: the swizzle of a row
+// depends on f*COLS + col.  With COLS = 2 (C = 2) the 4 frames of a row group get 4 distinct swizzles and one 8-row
+// phase of ldmatrix reads 8 distinct bank groups; with COLS = 4 (C = 4) only the frame's parity reaches the swizzle
+// and a phase reads each bank group twice - as many wavefronts as the LDS.32 of the previous layout, and the rows of
+// the tile stay 512 bytes long for the fetch.  The lane's row address only moves by a constant 8P*TILE bytes from one
+// ldmatrix to the next (immediate offsets, no address arithmetic).  Stage A's sample words
+// t*SS (t = 0..3) are four runs of 4 consecutive frames a quarter of the clip apart.
 using tma::mbar_expect_tx;
 using tma::mbar_init;
 using tma::mbar_wait;
 __device__ __forceinline__ void tma_load_2d(unsigned dst, const void* tmap, int c0, int c1, unsigned mbar) { tma::load_2d(dst, tmap, c0, c1, mbar); }
 
-// GQ: groups g < GQ are below Q = ceil(ceil(n/SPLIT)/4) for every n the variant is dispatched for
-template <int SPLIT, int G, int GQ, int SS, int WARPS, int CTAS>
+__device__ __forceinline__ void ldsm_x2_trans(unsigned addr, unsigned& r0, unsigned& r1, unsigned& r2, unsigned& r3) {
+  asm volatile("ldmatrix.sync.aligned.m16n16.x2.trans.shared.b8 {%0, %1, %2, %3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr) : "memory");
+}
+
+// shape of the tile: shared by the kernel and the tensor map of its launcher
+template <int C, int G, int WARPS>
+struct TmaTile {
+  static_assert(C == 2 || C == 4, "a warp owns 2 or 4 column blocks of 16 bytes");
+  static constexpr int P = 4 / C;                 // lanes that share an element
+  static constexpr int SEG = 16 * C;              // bytes of a frame one warp owns
+  static constexpr int TILE = WARPS * SEG;        // bytes of a frame one CTA owns
+  static constexpr int COLS = TILE / 128;         // 128-byte columns
+  static constexpr int ROWS = 8 * P * G;          // frames in the buffer: G ldmatrix.x2 of 8P frames each
+  static constexpr int row_boxes(int b) { return (ROWS % b == 0 && (ROWS / b) % 8 == 0 && ROWS / b <= 256) ? b : row_boxes(b + 1); }
+  static constexpr int BOX_ROWS = ROWS / row_boxes(1);   // <= 256 rows, a multiple of 8: every box starts on 1024 bytes
+  static constexpr int BYTES = ROWS * TILE;
+  static constexpr int SMEM = BYTES + 1024 + 16;  // + alignment of the buffer to 1024 bytes (the swizzle's period) + mbarrier, counter
+  static_assert(TILE % 128 == 0, "whole 128-byte columns");
+};
+
+// <C, G, SS, WARPS, CTAS>: C column blocks of 16 bytes per warp, 4G words per lane (2G per element), SS = stride of
+// the stage-A sample words (all real frames for every n the variant is dispatched for).
+template <int C, int G, int SS, int WARPS, int CTAS>
 __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const __grid_constant__ CUtensorMap tmap, uint8_t* __restrict__ out, int n,
                                                                           int ntiles) {
-  extern __shared__ __align__(128) uint8_t smem_tma[];
-  constexpr int LPS = 32 / SPLIT;
-  constexpr int SEG = LPS * 4;
-  constexpr int TILE = WARPS * SEG;          // bytes of a frame one CTA owns = pitch of the rows in shared memory
-  constexpr int ROWS = SPLIT * 4 * G;        // rows of the buffer (frames, the last ones past the clip)
-  constexpr unsigned BOX_BYTES = 4 * G * TILE;
+  extern __shared__ __align__(1024) uint8_t smem_tma[];
+  using T = TmaTile<C, G, WARPS>;
+  constexpr unsigned XMASK = 3u & ~(unsigned)(C - 1);   // lane bits of the quad members that share an element
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int part = lane / LPS, li = lane % LPS;
-  const int cnt0 = (n + SPLIT - 1) / SPLIT;
-  const int Q = (cnt0 + 3) >> 2;
-  const int delta = -(ROWS - n);
-  uint64_t* mbar_p = reinterpret_cast<uint64_t*>(smem_tma + ROWS * TILE);
+  const int delta = -(T::ROWS - n);
+  const unsigned sraw = (unsigned)__cvta_generic_to_shared(smem_tma);
+  const unsigned sdata = (sraw + 1023u) & ~1023u;
+  uint64_t* mbar_p = reinterpret_cast<uint64_t*>(smem_tma + (sdata - sraw) + T::BYTES);
   unsigned* count_p = reinterpret_cast<unsigned*>(mbar_p + 1);
   const unsigned mbar = (unsigned)__cvta_generic_to_shared(mbar_p);
-  const unsigned sdata = (unsigned)__cvta_generic_to_shared(smem_tma);
   auto fetch = [&](int tile) {   // one thread
-    mbar_expect_tx(mbar, SPLIT * BOX_BYTES);
+    mbar_expect_tx(mbar, T::BYTES);
 #pragma unroll
-    for (int b = 0; b < SPLIT; ++b) tma_load_2d(sdata + b * BOX_BYTES, &tmap, tile * (TILE > 256 ? TILE / 4 : TILE), b * 4 * G, mbar);
+    for (int r = 0; r < T::ROWS; r += T::BOX_ROWS) tma::load_3d(sdata + r * T::TILE, &tmap, 0, tile * T::COLS, r, mbar);
   };
   if (threadIdx.x == 0) {
     mbar_init(mbar, 1);
@@ -418,24 +478,26 @@ __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const 
   __syncthreads();
   int tile = blockIdx.x;
   if (threadIdx.x == 0 && tile < ntiles) fetch(tile);
-  // slot (g, r) of this lane: frame SPLIT*(r*Q + g) + part, row pitch TILE
-  const uint8_t* rowaddr[4];
-#pragma unroll
-  for (int r = 0; r < 4; ++r) rowaddr[r] = smem_tma + (SPLIT * (r * Q) + part) * TILE + warp * SEG + li * 4;
+  // the row this lane addresses: row rho of matrix M, which lands in quad member qq = rho >> 2 as frame
+  // 8Pj + f0 of column block qq % C
+  unsigned laddr;
+  {
+    const int rho = lane & 15, M = lane >> 4, qq = rho >> 2;
+    const int f0 = 8 * (qq / C) + 4 * ((M ^ qq) & 1) + (rho & 3);
+    const int byte = warp * T::SEG + 16 * (qq % C);   // of the tile
+    const int unit = f0 * T::COLS + (byte >> 7);
+    laddr = sdata + unit * 128 + ((((byte >> 4) & 7) ^ (unit & 7)) << 4);
+  }
+  // the two elements of this lane: bytes q%C*16 + (l>>2) + {0, 8} of the warp's segment; quad members q < C write them
+  const int q = lane & 3;
+  const int ebyte = warp * T::SEG + 16 * (q % C) + (lane >> 2);
   unsigned parity = 0;
   for (; tile < ntiles; tile += gridDim.x) {
     mbar_wait(mbar, parity);
     parity ^= 1;
     unsigned d[4 * G];
 #pragma unroll
-    for (int g = 0; g < G; ++g) {
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        d[4 * g + r] = 0;
-        if (g < GQ || g < Q) d[4 * g + r] = *reinterpret_cast<const unsigned*>(rowaddr[r] + g * (SPLIT * TILE));
-      }
-    }
-    transpose_groups<G>(d);   // consumes every load
+    for (int j = 0; j < G; ++j) ldsm_x2_trans(laddr + j * (8 * T::P * T::TILE), d[4 * j], d[4 * j + 1], d[4 * j + 2], d[4 * j + 3]);
     __syncwarp();
     if (lane == 0) {
       __threadfence_block();
@@ -446,8 +508,12 @@ __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const 
         fetch(tile + gridDim.x);
       }
     }
-    const unsigned res = sad_median<SPLIT, G, SS>(d, n, delta);
-    if (part == 0) reinterpret_cast<unsigned*>(out + ((long long)tile * WARPS + warp) * SEG)[li] = res;
+    const unsigned res = sad_median<2, XMASK, 2 * G, SS>(d, n, delta);
+    if (q < C) {
+      uint8_t* o = out + (long long)tile * T::TILE + ebyte;
+      o[0] = (uint8_t)res;
+      o[8] = (uint8_t)(res >> 8);
+    }
   }
 }
 

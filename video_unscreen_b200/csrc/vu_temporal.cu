@@ -12,7 +12,10 @@
 // the minimiser among 0..255 (see sad_search).  Frames are split over half /
 // quarter warps and the partial sums meet in a shuffle.  Unused slots are
 // padded with 0 on one side and 255 on the other, which keeps the middle order
-// statistics where they are.
+// statistics where they are.  That is the direct kernel; on 16-byte aligned
+// clips the TMA tile kernels run the same search on tiles staged in shared
+// memory and read them byte-transposed with ldmatrix, so their registers hold
+// 4 frames of one element without PRMT (vu_median_sad.cuh).
 //
 // n > 608: streaming 256-bin histograms in shared memory.  One warp owns a segment of
 // 32*PX consecutive bytes of every frame; lane l owns PX of them and a private
@@ -170,38 +173,39 @@ int launch_median_sad(const uint8_t* frames, int n, int64_t m, int64_t nseg, uin
   return record_cuda(cudaGetLastError());
 }
 
-// TMA tile kernels: the clip as a 2-D uint8 tensor [n][m], boxes of {TILE bytes, 4G frames}
+// TMA tile kernels: the clip as a 3-D tensor [n][m / 128][32] of 32-bit words, boxes of {TILE bytes, BOX_ROWS frames}
+// with the 128-byte swizzle (the layout is described in vu_median_sad.cuh).  Tiles only cover whole 128-byte units.
 using tma::encode_tiled_fn;
 using tma::EncodeTiledFn;
 
+// ntiles = groups of 8 segments to do (the kernel's tiles are TMA_WARPS segments);
 // pitch = bytes between consecutive frames of the (possibly subsampled) clip
-template <int SPLIT, int G, int GQ, int SS, int TMA_WARPS, int TMA_CTAS>
+template <int C, int G, int SS, int TMA_WARPS, int TMA_CTAS>
 int launch_median_sad_tma(const uint8_t* frames, int n, int64_t m, int64_t ntiles, uint8_t* out, vu_stream_t stream, int64_t pitch = 0) {
+  using T = msad::TmaTile<C, G, TMA_WARPS>;
+  static_assert(8 % TMA_WARPS == 0, "tiles of whole fractions of 8 segments");
+  ntiles *= 8 / TMA_WARPS;
   if (pitch == 0) pitch = m;
-  constexpr int TILE = TMA_WARPS * (128 / SPLIT);
-  constexpr int SMEM = SPLIT * 4 * G * TILE + 16;
-  constexpr bool U32 = TILE > 256;   // boxes are at most 256 elements wide: wide tiles are described in 32-bit words
-  static_assert(TILE <= 1024 && 4 * G <= 256, "TMA box limits");
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return VU_ERR_UNSUPPORTED;
   CUtensorMap tmap;
-  const cuuint64_t dims[2] = {(cuuint64_t)(U32 ? m / 4 : m), (cuuint64_t)n};
-  const cuuint64_t strides[1] = {(cuuint64_t)pitch};
-  const cuuint32_t box[2] = {(cuuint32_t)(U32 ? TILE / 4 : TILE), (cuuint32_t)(4 * G)};
-  const cuuint32_t estr[2] = {1, 1};
-  if (enc(&tmap, U32 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<uint8_t*>(frames), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+  const cuuint64_t dims[3] = {32, (cuuint64_t)(m / 128), (cuuint64_t)n};
+  const cuuint64_t strides[2] = {128, (cuuint64_t)pitch};
+  const cuuint32_t box[3] = {32, (cuuint32_t)T::COLS, (cuuint32_t)T::BOX_ROWS};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  if (enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t*>(frames), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
     return VU_ERR_UNSUPPORTED;
-  auto kernel = msad::median_sad_tma_kernel<SPLIT, G, GQ, SS, TMA_WARPS, TMA_CTAS>;
+  auto kernel = msad::median_sad_tma_kernel<C, G, SS, TMA_WARPS, TMA_CTAS>;
   static bool configured = false;
   if (!configured) {
-    int e = record_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    int e = record_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM));
     if (e) return e;
     configured = true;
   }
   const int64_t cap = (int64_t)device_sms() * TMA_CTAS;
   const int grid = (int)(ntiles < cap ? ntiles : cap);
-  kernel<<<grid, TMA_WARPS * 32, SMEM, S(stream)>>>(tmap, out, n, (int)ntiles);
+  kernel<<<grid, TMA_WARPS * 32, T::SMEM, S(stream)>>>(tmap, out, n, (int)ntiles);
   note_launch();
   return record_cuda(cudaGetLastError());
 }
@@ -524,9 +528,9 @@ int launch_median_two_pass(const uint8_t* frames, int n, int64_t m, int64_t nseg
   const int step = (n + 303) / 304;              // every step-th frame: at most 304 of them
   const int nsub = (n + step - 1) / step;
   int e;
-  if (nsub <= 152) e = launch_median_sad_tma<2, 19, 11, 2, 8, 2>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
-  else if (nsub <= 232) e = launch_median_sad_tma<2, 29, 20, 5, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
-  else e = launch_median_sad_tma<2, 38, 30, 8, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
+  if (nsub <= 152) e = launch_median_sad_tma<4, 19, 6, 8, 2>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
+  else if (nsub <= 232) e = launch_median_sad_tma<4, 29, 12, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
+  else e = launch_median_sad_tma<4, 38, 19, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
   if (e) return e;
   CUtensorMap tmap;
   const cuuint64_t dims[2] = {(cuuint64_t)(m / 4), (cuuint64_t)n};
@@ -597,15 +601,17 @@ extern "C" int vu_temporal_median_u8_ws(const uint8_t* frames, int n, int64_t m,
     // variant; SS = stride of the four sample groups of the estimate (all real frames over the n-range)
     // 16-byte aligned frame rows: persistent TMA tile kernels (8 adjacent segments per CTA, the next tile is fetched
     // while the current one is searched); segments that do not fill a tile go to the direct kernels below.
-    // <SPLIT, G, GQ, SS, warps per CTA (= segments per tile), CTAs per SM>
+    // <C, G, SS, warps per CTA (= segments per tile), CTAs per SM>: C column blocks of 16 bytes per warp (= seg / 16),
+    // 4G words per lane; SS = stride of the stage-A sample words, which hold frames below 8P(3SS/2 + 1) (P = 4/C):
+    // all real frames over the n-range of the variant
     const bool al16 = (reinterpret_cast<uintptr_t>(frames) % 16 == 0) && (m % 16 == 0);
     const int64_t ntiles = nseg / 8;
     if (al16 && path != 2 && n > 80 && ntiles > 0 && !g_median_direct) {
-      if (n <= 152) e = launch_median_sad_tma<2, 19, 11, 2, 8, 2>(frames, n, m, ntiles, out, stream);
-      else if (n <= 232) e = launch_median_sad_tma<2, 29, 20, 5, 8, 1>(frames, n, m, ntiles, out, stream);
-      else if (n <= 304) e = launch_median_sad_tma<2, 38, 30, 8, 8, 1>(frames, n, m, ntiles, out, stream);
-      else if (n <= 464) e = launch_median_sad_tma<4, 29, 20, 5, 8, 1>(frames, n, m, ntiles, out, stream);
-      else e = launch_median_sad_tma<4, 38, 30, 8, 8, 1>(frames, n, m, ntiles, out, stream);
+      if (n <= 152) e = launch_median_sad_tma<4, 19, 6, 8, 2>(frames, n, m, ntiles, out, stream);
+      else if (n <= 232) e = launch_median_sad_tma<4, 29, 12, 8, 1>(frames, n, m, ntiles, out, stream);
+      else if (n <= 304) e = launch_median_sad_tma<4, 38, 19, 8, 1>(frames, n, m, ntiles, out, stream);
+      else if (n <= 464) e = launch_median_sad_tma<2, 29, 12, 8, 1>(frames, n, m, ntiles, out, stream);
+      else e = launch_median_sad_tma<2, 38, 19, 8, 1>(frames, n, m, ntiles, out, stream);
       if (e == VU_OK) {
         const int64_t done = ntiles * 8;
         frames += done * seg;
