@@ -325,6 +325,43 @@ int vu_masked_temporal_mean(const uint8_t* frames, const uint8_t* masks, int n, 
 int vu_masked_temporal_mean_dilate32(const uint8_t* frames, const uint8_t* masks, int n, int h, int w, int min_count,
                                      uint8_t* bg_out, uint8_t* mask_always_out, vu_stream_t stream);
 
+/* Streamed temporal median: the clip is added in chunks, in any chunking and any order, and the finish writes the
+ * bytes vu_temporal_median_u8 writes for the whole clip (np.median(stack, 0).astype(u8)).  The state is
+ * vu_median_accum_bytes(m) bytes of device memory (512 per frame byte, rounded up to 128-byte tiles; 3.2 GB at 1080p,
+ * 12.7 GB at 4K), 16-byte aligned, whatever the clip length; its layout is private to these calls.
+ *   reset:  zero the state (an add with n_before == 0 overwrites it anyway, except an add captured into a CUDA graph,
+ *           which always accumulates: its replays add to whatever the state holds, and the caller counts them).
+ *   add:    frames [k][m] (any m, any alignment: 4-byte aligned rows with m % 4 == 0 take the vector loads); n_before
+ *           = frames added since the reset, tracked by the caller.  VU_ERR_INVALID_ARG, state untouched, when k < 1 or
+ *           n_before + k > 65535: the counters are 16 bits, so a state holds at most 65535 frames.
+ *   finish: out [m] = the median of the n frames added (1 <= n <= 65535): odd n order statistic (n + 1) / 2, even n
+ *           (s[n/2 - 1] + s[n/2]) >> 1.  The state is left as it was.
+ * Each add reads and writes the whole state (~1024 * m bytes) besides its k * m bytes of frames: add in chunks of
+ * hundreds of frames. */
+size_t vu_median_accum_bytes(int64_t m);
+int vu_median_accum_reset(void* state, int64_t m, vu_stream_t stream);
+int vu_median_accum_add_u8(void* state, int64_t m, const uint8_t* frames, int k, int n_before, vu_stream_t stream);
+int vu_median_accum_finish_u8(const void* state, int64_t m, int n, uint8_t* out, vu_stream_t stream);
+
+/* Streamed masked temporal mean, bg_offline.py:106-125 as the script runs it - a sum and a count accumulated frame by
+ * frame inside the read loop.  Any chunking and order gives the bytes of vu_masked_temporal_mean[_dilate32] on the
+ * whole clip.  State: vu_masked_mean_accum_bytes(h, w) = 16 bytes per pixel (uint32 sums of B, G, R and the count),
+ * 16-byte aligned, layout private; at most 16,000,000 frames in all (the sums are 32 bits).
+ *   add_dilate32: frames [k][h][w][3] and the RAW masks [k][h][w], dilate_mask(mask, 3, 2) (bg_offline.py:116) fused
+ *                 in as in vu_masked_temporal_mean_dilate32; w % 16 == 0 and 16-byte aligned frames / masks, else
+ *                 VU_ERR_UNSUPPORTED (dilate with vu_morph_u8, then add).
+ *   add:          the ALREADY DILATED masks [k][npix]; any npix and alignment.
+ *   finish:       bg_out [npix][3], mask_always_out [npix] as vu_masked_temporal_mean (255 where count <= min_count,
+ *                 bg 0 there).  The state is left as it was. */
+size_t vu_masked_mean_accum_bytes(int h, int w);
+int vu_masked_mean_accum_reset(void* state, int h, int w, vu_stream_t stream);
+int vu_masked_mean_accum_add_dilate32(void* state, const uint8_t* frames, const uint8_t* masks, int k, int h, int w,
+                                      vu_stream_t stream);
+int vu_masked_mean_accum_add(void* state, const uint8_t* frames, const uint8_t* masks_dilated, int k, int64_t npix,
+                             vu_stream_t stream);
+int vu_masked_mean_accum_finish(const void* state, int64_t npix, int min_count, uint8_t* bg_out, uint8_t* mask_always_out,
+                                vu_stream_t stream);
+
 /* One pass per frame of the bg_step live loop, tools/unscreen/bg_offline.py:154-160 + :171-172 (== bg.py:85-92, :99-100):
  * alpha = mask * (dilate_mask(g, 4, 2) // 255) with g = thresholded BGR2GRAY(|frame - bg|) (the difference gate of
  * vu_bgdiff_gate), fg = get_fg(frame, alpha, bgimg) with bgimg[alpha == 0] = frame[alpha == 0] (vu_get_fg with

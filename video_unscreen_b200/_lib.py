@@ -100,6 +100,15 @@ SIGNATURES = {
     "vu_temporal_median_u8_ws": (_i, [_p, _i, _i64, _p, _p, ctypes.c_size_t, _p]),
     "vu_masked_temporal_mean": (_i, [_p, _p, _i, _i64, _i, _p, _p, _p]),
     "vu_masked_temporal_mean_dilate32": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _p]),
+    "vu_median_accum_bytes": (_sz, [_i64]),
+    "vu_median_accum_reset": (_i, [_p, _i64, _p]),
+    "vu_median_accum_add_u8": (_i, [_p, _i64, _p, _i, _i, _p]),
+    "vu_median_accum_finish_u8": (_i, [_p, _i64, _i, _p, _p]),
+    "vu_masked_mean_accum_bytes": (_sz, [_i, _i]),
+    "vu_masked_mean_accum_reset": (_i, [_p, _i, _i, _p]),
+    "vu_masked_mean_accum_add_dilate32": (_i, [_p, _p, _p, _i, _i, _i, _p]),
+    "vu_masked_mean_accum_add": (_i, [_p, _p, _p, _i, _i64, _p]),
+    "vu_masked_mean_accum_finish": (_i, [_p, _i64, _i, _p, _p, _p]),
 }
 
 

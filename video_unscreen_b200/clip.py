@@ -126,6 +126,68 @@ def streamed(host_inputs, host_outputs, body, chunk, depth=2):
         st.synchronize()
 
 
+def _is_clip(x):
+    return isinstance(x, (np.ndarray, torch.Tensor))
+
+
+def _as_tensor(x):
+    return torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
+
+
+def _device_batch(b, dev):
+    """one batch [k, ...] of an iterable: a tensor or array, or a list of frames (what parallel_read_img returns)"""
+    if isinstance(b, (list, tuple)):
+        b = torch.stack([_as_tensor(x) for x in b])
+    b = _as_tensor(b)
+    return b if b.is_cuda else b.to(dev)
+
+
+def streamed_temporal_median(host_frames, chunk=256, depth=2, out=None):
+    """The exact temporal median (``ops.temporal_median``, byte for byte) of a clip that never has to be on the device in
+    one piece.  ``host_frames``: a clip [N, ...] in host memory (a pinned CPU tensor: the host->device copies of chunk i + 1
+    overlap the histogram add of chunk i; a numpy array or pageable tensor works too, with synchronous copies), or an
+    iterable of batches [k, ...] on the device (e.g. successive ``parallel_read_img(paths, on_device=True)`` results: the
+    clip then exists nowhere in full).  Device memory: the accumulator's 512 bytes per frame byte plus ``depth`` chunks.
+    At most 65535 frames.  Returns the median as a CUDA tensor of the frame's shape."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if _is_clip(host_frames):
+        t = _as_tensor(host_frames)
+        acc = ops.TemporalMedianAccumulator(t.shape[1:], dev)
+        streamed([t], [], lambda s, e, fr, outs: acc.add(fr), chunk, depth)
+    else:
+        acc = None
+        for b in host_frames:
+            b = _device_batch(b, dev)
+            if acc is None:
+                acc = ops.TemporalMedianAccumulator(b.shape[1:], dev)
+            acc.add(b)
+        if acc is None:
+            raise ValueError("streamed_temporal_median: no frames")
+    return acc.result(out)
+
+
+def streamed_masked_temporal_mean(host_frames, host_masks, chunk=256, ksize=3, iters=2, min_count=10, depth=2):
+    """bg_offline.py:106-125 (``ops.masked_temporal_mean_raw``, byte for byte) for a clip fed chunk by chunk:
+    ``host_frames`` [N,H,W,3] / ``host_masks`` [N,H,W] (raw masks) in host memory, copied to the device in chunks that
+    overlap the accumulation as in ``streamed_temporal_median``, or two iterables of device batches consumed in step.
+    Returns (bg [H,W,3], mask_always [H,W]) as CUDA tensors."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if _is_clip(host_frames):
+        f, mk = _as_tensor(host_frames), _as_tensor(host_masks)
+        acc = ops.MaskedMeanAccumulator(f.shape[1], f.shape[2], ksize, iters, min_count, dev)
+        streamed([f, mk], [], lambda s, e, fr, ms, outs: acc.add(fr, ms), chunk, depth)
+    else:
+        acc = None
+        for fb, mb in zip(host_frames, host_masks, strict=True):
+            fb, mb = _device_batch(fb, dev), _device_batch(mb, dev)
+            if acc is None:
+                acc = ops.MaskedMeanAccumulator(fb.shape[1], fb.shape[2], ksize, iters, min_count, dev)
+            acc.add(fb, mb)
+        if acc is None:
+            raise ValueError("streamed_masked_temporal_mean: no frames")
+    return acc.result()
+
+
 def cf_predict_clip(frames, segmasks, agent, chunk=64, out=None, streams=2, return_flags=False):
     """ColorFilteringAgent.forward(frame, mask, iters=0) for every frame of
     frames[N,H,W,3] / segmasks[N,H,W] with the agent's current mixtures

@@ -28,7 +28,10 @@
 // bins); even n returns (lo + hi) >> 1 like np.median(...).astype(uint8).
 //
 // vu_masked_temporal_mean: tools/unscreen/bg_offline.py:106-125 as integer
-// sums and counts per pixel, one float64 divide at the end.
+// sums and counts per pixel, one float64 divide at the end.  The
+// vu_masked_mean_accum_* calls keep those sums and counts in a state across
+// chunks of the clip (the fused-dilation kernel, templated on ACCUM) and share
+// the closed form of the end (mean_always / mean_byte).
 #include <cstdlib>
 
 #include "vu_common.cuh"
@@ -234,6 +237,15 @@ __global__ void __launch_bounds__(256) median_tail_kernel(const uint8_t* __restr
 }
 
 // ---- masked temporal mean -------------------------------------------------
+// bg_offline.py:121-125 for one pixel, shared by the resident kernels and the accumulator's finish:
+// mask_always = cnt <= min_count; bg = trunc(clip(sum / max(cnt, 1), 0, 255)), one float64 divide rounded once; 0
+// where always masked
+__device__ __forceinline__ bool mean_always(unsigned cnt, int min_count) { return cnt <= (unsigned)min_count; }
+__device__ __forceinline__ unsigned mean_byte(unsigned sum, unsigned cnt, bool always) {
+  const double q = fmin(fmax(__ddiv_rn((double)sum, (double)(cnt ? cnt : 1u)), 0.0), 255.0);
+  return always ? 0u : (unsigned)(int)q;
+}
+
 constexpr int TT = 256;
 __global__ void __launch_bounds__(TT) masked_mean_kernel(const uint8_t* __restrict__ frames, const uint8_t* __restrict__ masks, int n,
                                                          int64_t ngroups, int64_t npix, int min_count, uint8_t* __restrict__ bg_out,
@@ -269,13 +281,9 @@ __global__ void __launch_bounds__(TT) masked_mean_kernel(const uint8_t* __restri
     unsigned aw = 0;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      const bool always = cnt[i] <= (unsigned)min_count;
-      const double den = (double)(cnt[i] ? cnt[i] : 1u);
+      const bool always = mean_always(cnt[i], min_count);
 #pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        const double q = fmin(fmax(__ddiv_rn((double)sum[3 * i + k], den), 0.0), 255.0);
-        o[3 * i + k] = always ? 0 : (int)q;
-      }
+      for (int k = 0; k < 3; ++k) o[3 * i + k] = (int)mean_byte(sum[3 * i + k], cnt[i], always);
       aw |= (always ? 255u : 0u) << (8 * i);
     }
     unsigned w0, w1, w2;
@@ -326,13 +334,11 @@ __global__ void __launch_bounds__(TT) masked_mean16_kernel(const uint4* __restri
     for (int k = 0; k < 12; ++k) ow[k] = 0u;
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
-      const bool always = cnt[i] <= (unsigned)min_count;
-      const double den = (double)(cnt[i] ? cnt[i] : 1u);
+      const bool always = mean_always(cnt[i], min_count);
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
         const int b = 3 * i + k;
-        const double q = fmin(fmax(__ddiv_rn((double)sum[b], den), 0.0), 255.0);
-        ow[b >> 2] |= (always ? 0u : (unsigned)(int)q) << (8 * (b & 3));
+        ow[b >> 2] |= mean_byte(sum[b], cnt[i], always) << (8 * (b & 3));
       }
       aw[i >> 2] |= (always ? 255u : 0u) << (8 * (i & 3));
     }
@@ -363,9 +369,12 @@ __device__ __forceinline__ unsigned md_nibble(unsigned t) { return ((((t >> 7) &
 
 constexpr int MD_FPI = 6;   // frames per iteration (and per pair of barriers)
 
+// ACCUM: the sums and counts of these n frames are added to the accumulator state ({sum B, sum G, sum R, count} per
+// pixel) instead of being turned into the background
+template <bool ACCUM>
 __global__ void __launch_bounds__(256, 2) masked_mean_dilate_kernel(const uint8_t* __restrict__ frames, const uint8_t* __restrict__ masks, int n, int h,
                                                                   int w, int min_count, uint8_t* __restrict__ bg_out,
-                                                                  uint8_t* __restrict__ always_out) {
+                                                                  uint8_t* __restrict__ always_out, uint4* __restrict__ state) {
   // [stage: thresholded / dilated][frame of the iteration][plane][row][word]; plane 0: m == 255, plane 1: m >= 250
   __shared__ unsigned bits[2][MD_FPI][2][MD_ROWS][MD_PITCH];
   const int t = threadIdx.x;
@@ -479,20 +488,31 @@ __global__ void __launch_bounds__(256, 2) masked_mean_dilate_kernel(const uint8_
     if (f0 + MD_FPI < n) fetch_frames(f0 + MD_FPI);
   }
   if (!own) return;
+  const unsigned walked = (unsigned)((n + MD_FPI - 1) / MD_FPI * MD_FPI);   // frames of the walk, the padding ones included (never counted)
+  if (ACCUM) {
+    uint4* sp = state + (int64_t)oy * w + ox;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      uint4 s = sp[i];
+      s.x += sum[3 * i];
+      s.y += sum[3 * i + 1];
+      s.z += sum[3 * i + 2];
+      s.w += walked - cnt[i];
+      sp[i] = s;
+    }
+    return;
+  }
   unsigned ow[6], aw[2] = {0u, 0u};
 #pragma unroll
   for (int k = 0; k < 6; ++k) ow[k] = 0u;
-  const unsigned walked = (unsigned)((n + MD_FPI - 1) / MD_FPI * MD_FPI);   // frames of the walk, the padding ones included (never counted)
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const unsigned c = walked - cnt[i];
-    const bool always = c <= (unsigned)min_count;
-    const double den = (double)(c ? c : 1u);
+    const bool always = mean_always(c, min_count);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       const int b = 3 * i + k;
-      const double q = fmin(fmax(__ddiv_rn((double)sum[b], den), 0.0), 255.0);
-      ow[b >> 2] |= (always ? 0u : (unsigned)(int)q) << (8 * (b & 3));
+      ow[b >> 2] |= mean_byte(sum[b], c, always) << (8 * (b & 3));
     }
     aw[i >> 2] |= (always ? 255u : 0u) << (8 * (i & 3));
   }
@@ -500,6 +520,42 @@ __global__ void __launch_bounds__(256, 2) masked_mean_dilate_kernel(const uint8_
 #pragma unroll
   for (int k = 0; k < 3; ++k) bo[k] = make_uint2(ow[2 * k], ow[2 * k + 1]);
   *reinterpret_cast<uint2*>(always_out + (int64_t)oy * w + ox) = make_uint2(aw[0], aw[1]);
+}
+
+// ---- masked-mean accumulator: state = {sum B, sum G, sum R, count} per pixel (uint32 each) ----
+// k frames with ALREADY DILATED masks, any npix and alignment: one pixel per thread, byte loads
+__global__ void __launch_bounds__(TT) masked_mean_accum_add_kernel(uint4* __restrict__ state, const uint8_t* __restrict__ frames,
+                                                                   const uint8_t* __restrict__ masks, int k, int64_t npix) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < npix; p += stride) {
+    uint4 s = state[p];
+    const uint8_t* f = frames + 3 * p;
+    const uint8_t* mk = masks + p;
+#pragma unroll 4
+    for (int i = 0; i < k; ++i) {
+      const unsigned mv = __ldg(mk + (int64_t)i * npix);
+      const uint8_t* fp = f + (int64_t)i * 3 * npix;
+      const unsigned keep = mv == 255u ? 0u : 1u;   // frame * (1 - mask // 255)
+      s.x += __ldg(fp) * keep;
+      s.y += __ldg(fp + 1) * keep;
+      s.z += __ldg(fp + 2) * keep;
+      s.w += mv < 250u;                             // count += (mask < 250)
+    }
+    state[p] = s;
+  }
+}
+
+__global__ void __launch_bounds__(TT) masked_mean_accum_finish_kernel(const uint4* __restrict__ state, int64_t npix, int min_count,
+                                                                      uint8_t* __restrict__ bg_out, uint8_t* __restrict__ always_out) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < npix; p += stride) {
+    const uint4 s = state[p];
+    const bool always = mean_always(s.w, min_count);
+    bg_out[3 * p] = (uint8_t)mean_byte(s.x, s.w, always);
+    bg_out[3 * p + 1] = (uint8_t)mean_byte(s.y, s.w, always);
+    bg_out[3 * p + 2] = (uint8_t)mean_byte(s.z, s.w, always);
+    always_out[p] = always ? 255 : 0;
+  }
 }
 
 template <class P, int U>
@@ -661,7 +717,43 @@ extern "C" int vu_masked_temporal_mean_dilate32(const uint8_t* frames, const uin
     if (reinterpret_cast<uintptr_t>(p) & 15) return VU_ERR_UNSUPPORTED;
   if (w % 16 != 0 || (h + MD_TH - 1) / MD_TH > 65535) return VU_ERR_UNSUPPORTED;
   dim3 grid((w + MD_TW - 1) / MD_TW, (h + MD_TH - 1) / MD_TH);
-  masked_mean_dilate_kernel<<<grid, 256, 0, S(stream)>>>(frames, masks, n, h, w, min_count, bg_out, mask_always_out);
+  masked_mean_dilate_kernel<false><<<grid, 256, 0, S(stream)>>>(frames, masks, n, h, w, min_count, bg_out, mask_always_out, nullptr);
+  VU_RETURN_LAUNCH();
+}
+
+// 32-bit sums: 255 * (frames added) must fit, the caller keeps the total at most 16,000,000 frames
+extern "C" size_t vu_masked_mean_accum_bytes(int h, int w) { return (h > 0 && w > 0) ? (size_t)h * (size_t)w * 16 : 0; }
+
+extern "C" int vu_masked_mean_accum_reset(void* state, int h, int w, vu_stream_t stream) {
+  VU_REQUIRE(state && h > 0 && w > 0);
+  return record_cuda(cudaMemsetAsync(state, 0, vu_masked_mean_accum_bytes(h, w), S(stream)));
+}
+
+extern "C" int vu_masked_mean_accum_add_dilate32(void* state, const uint8_t* frames, const uint8_t* masks, int k, int h, int w, vu_stream_t stream) {
+  VU_REQUIRE(state && frames && masks && k >= 1 && h > 0 && w > 0);
+  VU_REQUIRE((reinterpret_cast<uintptr_t>(state) & 15) == 0);
+  if (k > 16000000) return VU_ERR_UNSUPPORTED;
+  if (((reinterpret_cast<uintptr_t>(frames) | reinterpret_cast<uintptr_t>(masks)) & 15) != 0) return VU_ERR_UNSUPPORTED;
+  if (w % 16 != 0 || (h + MD_TH - 1) / MD_TH > 65535) return VU_ERR_UNSUPPORTED;
+  dim3 grid((w + MD_TW - 1) / MD_TW, (h + MD_TH - 1) / MD_TH);
+  masked_mean_dilate_kernel<true><<<grid, 256, 0, S(stream)>>>(frames, masks, k, h, w, 0, nullptr, nullptr, static_cast<uint4*>(state));
+  VU_RETURN_LAUNCH();
+}
+
+extern "C" int vu_masked_mean_accum_add(void* state, const uint8_t* frames, const uint8_t* masks_dilated, int k, int64_t npix, vu_stream_t stream) {
+  VU_REQUIRE(state && frames && masks_dilated && k >= 1 && npix > 0);
+  VU_REQUIRE((reinterpret_cast<uintptr_t>(state) & 15) == 0);
+  if (k > 16000000) return VU_ERR_UNSUPPORTED;
+  masked_mean_accum_add_kernel<<<grid_for(npix, TT, 8), TT, 0, S(stream)>>>(static_cast<uint4*>(state), frames, masks_dilated, k, npix);
+  VU_RETURN_LAUNCH();
+}
+
+extern "C" int vu_masked_mean_accum_finish(const void* state, int64_t npix, int min_count, uint8_t* bg_out, uint8_t* mask_always_out,
+                                           vu_stream_t stream) {
+  VU_REQUIRE(state && bg_out && mask_always_out && npix > 0);
+  VU_REQUIRE((reinterpret_cast<uintptr_t>(state) & 15) == 0);
+  masked_mean_accum_finish_kernel<<<grid_for(npix, TT, 8), TT, 0, S(stream)>>>(static_cast<const uint4*>(state), npix, min_count, bg_out,
+                                                                               mask_always_out);
   VU_RETURN_LAUNCH();
 }
 

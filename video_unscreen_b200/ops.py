@@ -637,6 +637,101 @@ def masked_temporal_mean_raw(frames, masks, ksize=3, iters=2, min_count=10):
     return masked_temporal_mean(frames, dilate(masks, ksize, iters), min_count)
 
 
+MEDIAN_ACCUM_MAX_FRAMES = 65535      # 16-bit histogram counters
+MEAN_ACCUM_MAX_FRAMES = 16000000     # 32-bit sums of bytes
+
+
+class TemporalMedianAccumulator:
+    """The exact temporal median of a clip that arrives in chunks: ``add`` any number of batches [k, *frame_shape], in any
+    order, then ``result()`` is ``temporal_median`` of all of them together, byte for byte.  The state is 512 bytes per frame
+    byte (3.2 GB at 1080p, 12.7 GB at 4K) whatever the clip length; at most 65535 frames.  Every call enqueues on the
+    current stream and neither allocates device memory (except ``result``'s output) nor synchronises, so an ``add`` can
+    run on a side stream or inside a CUDA graph.  A captured add always accumulates into the state, whatever ``.n`` was at
+    capture.  ``.n`` is counted on the host when ``add`` is called, so it does not see replays, and the 65535-frame limit
+    is not checked for them: after replaying a captured add of k frames r times, add r * k to ``.n`` (a plain attribute)
+    before ``result()``, and keep the total at most 65535.  Each add reads and writes the whole state: chunks of hundreds
+    of frames."""
+
+    def __init__(self, frame_shape, device=None):
+        self.frame_shape = tuple(int(s) for s in frame_shape)
+        self.m = int(np.prod(self.frame_shape, dtype=np.int64))
+        self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        nbytes = int(lib().vu_median_accum_bytes(self.m))
+        self.state = torch.empty(max(nbytes, 16), dtype=u8, device=self.device)
+        self.reset()
+
+    def reset(self):
+        check(lib().vu_median_accum_reset(_p(self.state), self.m, _stream()))
+        self.n = 0
+
+    def add(self, frames):
+        frames = _dev(frames)
+        if tuple(frames.shape[1:]) != self.frame_shape:
+            raise ValueError(f"expected frames [k, {self.frame_shape}], got {tuple(frames.shape)}")
+        k = frames.shape[0]
+        if k == 0:
+            return self
+        rc = lib().vu_median_accum_add_u8(_p(self.state), self.m, _p(frames), k, self.n, _stream())
+        if rc != _lib.VU_OK and self.n + k > MEDIAN_ACCUM_MAX_FRAMES:     # refused, the state untouched
+            raise _lib.VuError(f"the median accumulator holds at most {MEDIAN_ACCUM_MAX_FRAMES} frames: {self.n} + {k}")
+        check(rc)
+        self.n += k
+        return self
+
+    def result(self, out=None):
+        if out is None:
+            out = torch.empty(self.frame_shape, dtype=u8, device=self.device)
+        elif not (out.is_cuda and out.dtype == u8 and out.is_contiguous() and out.numel() == self.m):
+            raise ValueError(f"out must be a contiguous CUDA uint8 tensor of {self.m} bytes")
+        check(lib().vu_median_accum_finish_u8(_p(self.state), self.m, self.n, _p(out), _stream()))
+        return out
+
+
+class MaskedMeanAccumulator:
+    """bg_offline.py:106-125 for a clip that arrives in chunks: ``add(frames [k,h,w,3], masks [k,h,w])`` with the RAW masks
+    (dilated by dilate_mask(mask, ksize, iters) like ``masked_temporal_mean_raw``), in any chunking and order; ``result()``
+    returns (bg [h,w,3], mask_always [h,w]), byte for byte those of ``masked_temporal_mean_raw`` on the whole clip.  16 bytes
+    of state per pixel.  Enqueues on the current stream; nothing synchronises."""
+
+    def __init__(self, h, w, ksize=3, iters=2, min_count=10, device=None):
+        self.h, self.w = int(h), int(w)
+        self.ksize, self.iters, self.min_count = int(ksize), int(iters), int(min_count)
+        self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        self.state = torch.empty(int(lib().vu_masked_mean_accum_bytes(self.h, self.w)), dtype=u8, device=self.device)
+        self.reset()
+
+    def reset(self):
+        check(lib().vu_masked_mean_accum_reset(_p(self.state), self.h, self.w, _stream()))
+        self.n = 0
+
+    def add(self, frames, masks):
+        frames, masks = _img(frames), _mask(masks)
+        k = frames.shape[0]
+        if frames.shape != (k, self.h, self.w, 3) or masks.shape != (k, self.h, self.w):
+            raise ValueError(f"expected frames [k,{self.h},{self.w},3] and masks [k,{self.h},{self.w}], got {tuple(frames.shape)}, {tuple(masks.shape)}")
+        if k == 0:
+            return self
+        if self.n + k > MEAN_ACCUM_MAX_FRAMES:
+            raise _lib.VuError(f"the masked-mean accumulator holds at most {MEAN_ACCUM_MAX_FRAMES} frames: {self.n} + {k}")
+        rc = _lib.ERR_UNSUPPORTED
+        if (self.ksize, self.iters) == (3, 2):
+            rc = lib().vu_masked_mean_accum_add_dilate32(_p(self.state), _p(frames), _p(masks), k, self.h, self.w, _stream())
+        if rc == _lib.ERR_UNSUPPORTED:
+            d = dilate(masks, self.ksize, self.iters)
+            rc = lib().vu_masked_mean_accum_add(_p(self.state), _p(frames), _p(d), k, self.h * self.w, _stream())
+        check(rc)
+        self.n += k
+        return self
+
+    def result(self):
+        if self.n < 1:
+            raise _lib.VuError("the masked-mean accumulator holds no frames")
+        bg = torch.empty((self.h, self.w, 3), dtype=u8, device=self.device)
+        always = torch.empty((self.h, self.w), dtype=u8, device=self.device)
+        check(lib().vu_masked_mean_accum_finish(_p(self.state), self.h * self.w, self.min_count, _p(bg), _p(always), _stream()))
+        return bg, always
+
+
 # ---- per-frame branches on the device (batched clips) --------------------------------
 
 def cf_samples(hsv_lo, mask_lo, mask_op, max_samples, prior=None, invert=False):
