@@ -581,6 +581,26 @@ def regionfill(I, mask, factor=1.0):
     return out
 
 
+def laplace_residual(x, I, mask):
+    """max |nn x[p] - sum of x over p's in-image 4-neighbours| over the masked pixels p (float64): how far a filled plane x
+    is from solving regionfill's Laplace system (factor 1.0), without assembling or solving it.  Outside the mask the
+    boundary data I is used, so x only has to be right under the mask.  x, I: [H,W] or [C,H,W] planes sharing mask [H,W]."""
+    m = np.asarray(mask) != 0
+    y = np.where(m, np.asarray(x, np.float64), np.asarray(I, np.float64))
+    if not m.any():
+        return 0.0
+    nb = np.zeros_like(y)
+    nb[..., 1:, :] += y[..., :-1, :]
+    nb[..., :-1, :] += y[..., 1:, :]
+    nb[..., :, 1:] += y[..., :, :-1]
+    nb[..., :, :-1] += y[..., :, 1:]
+    h, w = m.shape
+    nn = np.full((h, w), 4.0)
+    nn[[0, -1], :] -= 1
+    nn[:, [0, -1]] -= 1
+    return float(np.abs(nn * y - nb)[..., m].max())
+
+
 def bg_by_regionfill(img_hsv, mask, boundary_ksize=7, boundary_iters=10):
     """BackgroundAgent.get_bg_by_regionfill, unscreen/bgmodel/agent.py:133-157: V from regionfill at half resolution,
     H and S from the boundary's mean colour."""

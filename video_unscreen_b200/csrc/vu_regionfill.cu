@@ -268,13 +268,15 @@ extern "C" int vu_regionfill_f64(double* x, const uint8_t* mask, int planes, int
     if (e) return e;
     done = true;
     worst = 0.0;
+    bool nan = false;
     for (int c = 0; c < planes; ++c) {
       const double rr = host[c].rr[k % 3], bb = host[c].bb;
-      if (!(rr <= tol * tol * bb)) done = false;      // a NaN keeps iterating until max_iters
+      if (!(rr <= tol * tol * bb)) done = false;
+      nan |= rr != rr;
       const double rel = bb > 0.0 ? sqrt(rr / bb) : (rr > 0.0 ? INFINITY : 0.0);
       if (!(rel <= worst)) worst = rel;
     }
-    if (done || k >= max_iters) break;
+    if (done || nan || k >= max_iters) break;      // a NaN (non-finite input) stops at once and is reported as the residual
     const int upto = k + CHECK < max_iters ? k + CHECK : max_iters;
     note_launch(2 * (upto - k));
     for (; k < upto; ++k) {

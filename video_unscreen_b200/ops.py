@@ -871,11 +871,13 @@ def resize_linear_f64(x, dh, dw, fx=None, fy=None, keep_mask=None, keep_src=None
     return out
 
 
-def laplace_fill(planes, mask, tol=1e-10, max_iters=50000, snap_eps=1e-6):
+def laplace_fill(planes, mask, tol=1e-10, max_iters=None, snap_eps=1e-6):
     """regionfillLaplace (utils/region_fill.py:26-63) for float64 planes [C,H,W] sharing mask [H,W] (> 0 = fill): solved on
     the mask's bounding box (+ 1 pixel, so that only real image borders act as borders).  -> (filled planes, iterations).
     Filled values within ``snap_eps`` of an integer are set to it (the callers truncate to uint8; include/vu_b200.h).
-    Raises if the conjugate gradients did not reach ``tol`` (relative residual) within ``max_iters``."""
+    Raises if the conjugate gradients did not reach ``tol`` (relative residual) within ``max_iters``, by default the
+    number of pixels in that box (at least 50000): in exact arithmetic CG ends within as many iterations as there are
+    unknowns, so a valid mask of any size gets a cap it cannot need."""
     planes, mask = _dev(planes, torch.float64), _mask(mask)
     c, h, w = planes.shape
     if tuple(mask.shape) != (h, w):
@@ -889,6 +891,8 @@ def laplace_fill(planes, mask, tol=1e-10, max_iters=50000, snap_eps=1e-6):
     x = out[:, r0:r1, c0:c1].contiguous()
     m = mask[r0:r1, c0:c1].contiguous()
     rh, rw = r1 - r0, c1 - c0
+    if max_iters is None:
+        max_iters = max(50000, rh * rw)
     nbytes = lib().vu_regionfill_workspace_bytes(c, rh, rw)
     ws = torch.empty(nbytes, dtype=u8, device=planes.device)
     iters, resid = ctypes.c_int32(0), ctypes.c_double(0.0)
