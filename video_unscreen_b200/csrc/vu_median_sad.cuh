@@ -399,8 +399,10 @@ __global__ void __launch_bounds__(128, CTAS) median_sad_kernel(const uint8_t* __
 //
 // Measured on the B200 (tools/ldgsts_ubench.cu, fetch only): "one row per frame" streams at 2.8 TB/s when a warp
 // fetches 64-byte rows on its own, at 5.9 TB/s with 128-byte rows and at 7.2 TB/s with 512-byte rows: requests must
-// cover whole 128-byte lines, and the direct kernel above (64 bytes per frame and warp) cannot get there.  Here a CTA
-// of WARPS warps owns tiles of WARPS adjacent segments of 16*C bytes (8 warps, C = 4: 512 bytes of every frame).  The
+// cover whole 128-byte lines, and the direct kernel above (64 bytes per frame and warp) cannot get there.  Here a
+// pipeline of WARPS warps owns tiles of WARPS adjacent segments of 16*C bytes (4 warps at C = 4 or 8 warps at C = 2: 256
+// bytes of every frame).  For n <= 304 one CTA per SM runs 2 to 4 such pipelines, each with its own buffer, mbarrier
+// and counter; their loops drift apart, so one pipeline drains and refills while another searches.  The
 // clip is described to the TMA unit as a 3-D tensor [n frames][m/128 chunks][128 bytes], and boxes of {TILE bytes x
 // BOX_ROWS frames} (cp.async.bulk.tensor.3d with the 128-byte swizzle, one elected thread, completion counted in bytes
 // on an mbarrier) bring the tile into shared memory as rows of TILE bytes.  The swizzle works on 128-byte units: unit
@@ -419,10 +421,9 @@ __global__ void __launch_bounds__(128, CTAS) median_sad_kernel(const uint8_t* __
 // element are dealt to the P = 4/C quad members q, q+C, ..: with C = 4 one lane holds every frame of its two elements
 // and S needs no shuffle; with C = 2 two lanes hold half the frames each (shfl_xor 2).  Word k = 2j+M (matrix M of the
 // j-th ldmatrix.x2) of quad member q holds frames 8Pj + 8(q/C) + 4((M^q)&1) + 0..3.  Banks: the swizzle of a row
-// depends on f*COLS + col.  With COLS = 2 (C = 2) the 4 frames of a row group get 4 distinct swizzles and one 8-row
-// phase of ldmatrix reads 8 distinct bank groups; with COLS = 4 (C = 4) only the frame's parity reaches the swizzle
-// and a phase reads each bank group twice - as many wavefronts as the LDS.32 of the previous layout, and the rows of
-// the tile stay 512 bytes long for the fetch.  The lane's row address only moves by a constant 8P*TILE bytes from one
+// depends on f*COLS + col.  With COLS = TILE/128 = 2 the 4 frames of a row group get 4 distinct swizzles and one 8-row
+// phase of ldmatrix reads 8 distinct bank groups (C = 4 and C = 2 alike); with 512-byte tiles (COLS = 4) only the
+// frame's parity would reach the swizzle and a phase would read each bank group twice.  The lane's row address only moves by a constant 8P*TILE bytes from one
 // ldmatrix to the next (immediate offsets, no address arithmetic).  Stage A's sample words
 // t*SS (t = 0..3) are four runs of 4 consecutive frames a quarter of the clip apart.
 using tma::mbar_expect_tx;
@@ -446,23 +447,41 @@ struct TmaTile {
   static constexpr int row_boxes(int b) { return (ROWS % b == 0 && (ROWS / b) % 8 == 0 && ROWS / b <= 256) ? b : row_boxes(b + 1); }
   static constexpr int BOX_ROWS = ROWS / row_boxes(1);   // <= 256 rows, a multiple of 8: every box starts on 1024 bytes
   static constexpr int BYTES = ROWS * TILE;
-  static constexpr int SMEM = BYTES + 1024 + 16;  // + alignment of the buffer to 1024 bytes (the swizzle's period) + mbarrier, counter
+  // PIPES buffers + alignment to 1024 bytes (the swizzle's period) + an mbarrier and a counter per buffer
+  static constexpr int smem(int pipes) { return pipes * BYTES + 1024 + 16 * pipes; }
   static_assert(TILE % 128 == 0, "whole 128-byte columns");
 };
 
-// <C, G, SS, WARPS, CTAS>: C column blocks of 16 bytes per warp, 4G words per lane (2G per element), SS = stride of
-// the stage-A sample words (all real frames for every n the variant is dispatched for).
-template <int C, int G, int SS, int WARPS, int CTAS>
-__global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const __grid_constant__ CUtensorMap tmap, uint8_t* __restrict__ out, int n,
-                                                                          int ntiles) {
+// Timeline of the tile loop (TRACE kernels only, tools/median_timeline.py): one record of TRACE_WORDS words per warp
+// and tile it searched, at trace[((pipeline * WARPS + warp) * ceil(ntiles / pipelines) + k) * TRACE_WORDS] for its
+// k-th tile: %globaltimer (ns) when the mbarrier wait begins, when it ends, when the warp's ldmatrix results have
+// arrived, when the search ends and when this warp issued the refill (0 if another warp did), then
+// %smid << 40 | (%warpid & 63) << 32 | a
+// word of the drained data (stored so that the drain stamp has to wait for the data).
+constexpr int TRACE_WORDS = 6;
+__device__ __forceinline__ unsigned long long globaltimer() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)::"memory");
+  return t;
+}
+
+// <C, G, SS, WARPS, CTAS, PIPES>: C column blocks of 16 bytes per warp, 4G words per lane (2G per element), SS = stride
+// of the stage-A sample words (all real frames for every n the variant is dispatched for).  A CTA runs PIPES independent
+// pipelines of WARPS warps, each with its own tile buffer, mbarrier and refill counter (pipeline p of CTA b is pipeline
+// b * PIPES + p of the grid).  TRACE: record the timeline above into `trace` (off in the library; `trace` is unused then).
+template <int C, int G, int SS, int WARPS, int CTAS, int PIPES = 1, bool TRACE = false>
+__global__ void __launch_bounds__(PIPES * WARPS * 32, CTAS) median_sad_tma_kernel(const __grid_constant__ CUtensorMap tmap, uint8_t* __restrict__ out,
+                                                                                  int n, int ntiles, unsigned long long* __restrict__ trace) {
   extern __shared__ __align__(1024) uint8_t smem_tma[];
   using T = TmaTile<C, G, WARPS>;
+  static_assert(T::BYTES % 1024 == 0, "every pipeline's buffer starts on the swizzle's period");
   constexpr unsigned XMASK = 3u & ~(unsigned)(C - 1);   // lane bits of the quad members that share an element
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31, pipe = (threadIdx.x >> 5) / WARPS, warp = (threadIdx.x >> 5) % WARPS;
   const int delta = -(T::ROWS - n);
   const unsigned sraw = (unsigned)__cvta_generic_to_shared(smem_tma);
-  const unsigned sdata = (sraw + 1023u) & ~1023u;
-  uint64_t* mbar_p = reinterpret_cast<uint64_t*>(smem_tma + (sdata - sraw) + T::BYTES);
+  const unsigned sbase = (sraw + 1023u) & ~1023u;
+  const unsigned sdata = sbase + pipe * T::BYTES;
+  uint64_t* mbar_p = reinterpret_cast<uint64_t*>(smem_tma + (sbase - sraw) + PIPES * T::BYTES) + 2 * pipe;
   unsigned* count_p = reinterpret_cast<unsigned*>(mbar_p + 1);
   const unsigned mbar = (unsigned)__cvta_generic_to_shared(mbar_p);
   auto fetch = [&](int tile) {   // one thread
@@ -470,14 +489,15 @@ __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const 
 #pragma unroll
     for (int r = 0; r < T::ROWS; r += T::BOX_ROWS) tma::load_3d(sdata + r * T::TILE, &tmap, 0, tile * T::COLS, r, mbar);
   };
-  if (threadIdx.x == 0) {
+  if (warp == 0 && lane == 0) {
     mbar_init(mbar, 1);
     *count_p = 0;
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-  int tile = blockIdx.x;
-  if (threadIdx.x == 0 && tile < ntiles) fetch(tile);
+  const int npipes = gridDim.x * PIPES;
+  int tile = blockIdx.x * PIPES + pipe;
+  if (warp == 0 && lane == 0 && tile < ntiles) fetch(tile);
   // the row this lane addresses: row rho of matrix M, which lands in quad member qq = rho >> 2 as frame
   // 8Pj + f0 of column block qq % C
   unsigned laddr;
@@ -492,20 +512,35 @@ __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const 
   const int q = lane & 3;
   const int ebyte = warp * T::SEG + 16 * (q % C) + (lane >> 2);
   unsigned parity = 0;
-  for (; tile < ntiles; tile += gridDim.x) {
+  unsigned long long* rec = nullptr;
+  if constexpr (TRACE) rec = trace + (long long)((blockIdx.x * PIPES + pipe) * WARPS + warp) * ((ntiles + npipes - 1) / npipes) * TRACE_WORDS;
+  for (; tile < ntiles; tile += npipes) {
+    unsigned long long t_wait = 0, t_ready = 0, t_drained = 0, t_refill = 0;
+    if constexpr (TRACE) t_wait = globaltimer();
     mbar_wait(mbar, parity);
     parity ^= 1;
+    if constexpr (TRACE) t_ready = globaltimer();
     unsigned d[4 * G];
 #pragma unroll
     for (int j = 0; j < G; ++j) ldsm_x2_trans(laddr + j * (8 * T::P * T::TILE), d[4 * j], d[4 * j + 1], d[4 * j + 2], d[4 * j + 3]);
+    if constexpr (TRACE) {
+      if (lane == 0) {
+        unsigned smid, hwarp;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        asm volatile("mov.u32 %0, %%warpid;" : "=r"(hwarp));
+        rec[5] = (unsigned long long)smid << 40 | (unsigned long long)(hwarp & 63) << 32 | (d[0] ^ d[4 * G - 1]);
+      }
+      t_drained = globaltimer();
+    }
     __syncwarp();
     if (lane == 0) {
       __threadfence_block();
       const unsigned old = atomicAdd(count_p, 1u);
-      if (old % WARPS == WARPS - 1 && tile + (int)gridDim.x < ntiles) {
+      if (old % WARPS == WARPS - 1 && tile + npipes < ntiles) {
         __threadfence_block();
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        fetch(tile + gridDim.x);
+        fetch(tile + npipes);
+        if constexpr (TRACE) t_refill = globaltimer();
       }
     }
     const unsigned res = sad_median<2, XMASK, 2 * G, SS>(d, n, delta);
@@ -513,6 +548,17 @@ __global__ void __launch_bounds__(WARPS * 32, CTAS) median_sad_tma_kernel(const 
       uint8_t* o = out + (long long)tile * T::TILE + ebyte;
       o[0] = (uint8_t)res;
       o[8] = (uint8_t)(res >> 8);
+    }
+    if constexpr (TRACE) {
+      const unsigned long long t_done = globaltimer();
+      if (lane == 0) {
+        rec[0] = t_wait;
+        rec[1] = t_ready;
+        rec[2] = t_drained;
+        rec[3] = t_done;
+        rec[4] = t_refill;
+      }
+      rec += TRACE_WORDS;
     }
   }
 }

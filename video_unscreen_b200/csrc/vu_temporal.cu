@@ -181,13 +181,16 @@ int launch_median_sad(const uint8_t* frames, int n, int64_t m, int64_t nseg, uin
 using tma::encode_tiled_fn;
 using tma::EncodeTiledFn;
 
-// ntiles = groups of 8 segments to do (the kernel's tiles are TMA_WARPS segments);
-// pitch = bytes between consecutive frames of the (possibly subsampled) clip
-template <int C, int G, int SS, int TMA_WARPS, int TMA_CTAS>
-int launch_median_sad_tma(const uint8_t* frames, int n, int64_t m, int64_t ntiles, uint8_t* out, vu_stream_t stream, int64_t pitch = 0) {
+// Does the whole tiles (TMA_WARPS segments of 16C bytes each) of the first nseg segments and sets *done to the number
+// of segments they cover; the rest is the caller's.  pitch = bytes between consecutive frames of the (possibly
+// subsampled) clip.  TRACE kernels record their timeline into `trace` (see vu_median_sad.cuh).
+template <int C, int G, int SS, int TMA_WARPS, int TMA_CTAS, int PIPES = 1, bool TRACE = false>
+int launch_median_sad_tma(const uint8_t* frames, int n, int64_t m, int64_t nseg, uint8_t* out, vu_stream_t stream, int64_t* done, int64_t pitch = 0,
+                          unsigned long long* trace = nullptr) {
   using T = msad::TmaTile<C, G, TMA_WARPS>;
-  static_assert(8 % TMA_WARPS == 0, "tiles of whole fractions of 8 segments");
-  ntiles *= 8 / TMA_WARPS;
+  const int64_t ntiles = nseg / TMA_WARPS;
+  *done = 0;
+  if (ntiles == 0) return VU_OK;
   if (pitch == 0) pitch = m;
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return VU_ERR_UNSUPPORTED;
@@ -199,18 +202,21 @@ int launch_median_sad_tma(const uint8_t* frames, int n, int64_t m, int64_t ntile
   if (enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t*>(frames), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
     return VU_ERR_UNSUPPORTED;
-  auto kernel = msad::median_sad_tma_kernel<C, G, SS, TMA_WARPS, TMA_CTAS>;
+  auto kernel = msad::median_sad_tma_kernel<C, G, SS, TMA_WARPS, TMA_CTAS, PIPES, TRACE>;
+  constexpr int smem = T::smem(PIPES);
   static bool configured = false;
   if (!configured) {
-    int e = record_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM));
+    int e = record_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     if (e) return e;
     configured = true;
   }
-  const int64_t cap = (int64_t)device_sms() * TMA_CTAS;
-  const int grid = (int)(ntiles < cap ? ntiles : cap);
-  kernel<<<grid, TMA_WARPS * 32, T::SMEM, S(stream)>>>(tmap, out, n, (int)ntiles);
+  const int64_t cap = (int64_t)device_sms() * TMA_CTAS, need = (ntiles + PIPES - 1) / PIPES;
+  const int grid = (int)(need < cap ? need : cap);
+  kernel<<<grid, PIPES * TMA_WARPS * 32, smem, S(stream)>>>(tmap, out, n, (int)ntiles, trace);
   note_launch();
-  return record_cuda(cudaGetLastError());
+  const int e = record_cuda(cudaGetLastError());
+  if (e == VU_OK) *done = ntiles * TMA_WARPS;
+  return e;
 }
 
 // elements that do not fill a whole segment (and unaligned inputs): one CTA
@@ -583,10 +589,12 @@ int launch_median_two_pass(const uint8_t* frames, int n, int64_t m, int64_t nseg
   if (ntiles == 0 || ntiles > 0x7fffffff) return VU_ERR_UNSUPPORTED;
   const int step = (n + 303) / 304;              // every step-th frame: at most 304 of them
   const int nsub = (n + step - 1) / step;
+  const int64_t nsub_seg = ntiles * msad::RF_WARPS;   // the segments pass 2 refines: whole tiles of the subsample pass too
+  int64_t done;                                       // = nsub_seg
   int e;
-  if (nsub <= 152) e = launch_median_sad_tma<4, 19, 6, 8, 2>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
-  else if (nsub <= 232) e = launch_median_sad_tma<4, 29, 12, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
-  else e = launch_median_sad_tma<4, 38, 19, 8, 1>(frames, nsub, m, ntiles, out, stream, (int64_t)step * m);
+  if (nsub <= 152) e = launch_median_sad_tma<4, 19, 6, 4, 1, 4>(frames, nsub, m, nsub_seg, out, stream, &done, (int64_t)step * m);
+  else if (nsub <= 232) e = launch_median_sad_tma<4, 29, 12, 4, 1, 3>(frames, nsub, m, nsub_seg, out, stream, &done, (int64_t)step * m);
+  else e = launch_median_sad_tma<4, 38, 19, 4, 1, 2>(frames, nsub, m, nsub_seg, out, stream, &done, (int64_t)step * m);
   if (e) return e;
   CUtensorMap tmap;
   const cuuint64_t dims[2] = {(cuuint64_t)(m / 4), (cuuint64_t)n};
@@ -609,7 +617,6 @@ int launch_median_two_pass(const uint8_t* frames, int n, int64_t m, int64_t nseg
   e = record_cuda(cudaGetLastError());
   if (e) return e;
   // segments that do not fill a tile are flagged wholesale; the histogram kernel then redoes every flagged segment
-  const int64_t done = ntiles * msad::RF_WARPS;
   if (done < nseg) {
     e = record_cuda(cudaMemsetAsync(flags + done, 1, (size_t)(nseg - done), S(stream)));
     if (e) return e;
@@ -655,21 +662,22 @@ extern "C" int vu_temporal_median_u8_ws(const uint8_t* frames, int n, int64_t m,
     // <SPLIT, G, GFULL, SS, CTAs/SM>: G = register groups of 4 frames per lane, the smallest variant that holds
     // ceil(n / SPLIT) frames; GFULL = groups whose first three rows are real frames over the whole n-range of the
     // variant; SS = stride of the four sample groups of the estimate (all real frames over the n-range)
-    // 16-byte aligned frame rows: persistent TMA tile kernels (8 adjacent segments per CTA, the next tile is fetched
-    // while the current one is searched); segments that do not fill a tile go to the direct kernels below.
-    // <C, G, SS, warps per CTA (= segments per tile), CTAs per SM>: C column blocks of 16 bytes per warp (= seg / 16),
+    // 16-byte aligned frame rows: persistent TMA tile kernels (a pipeline of warps owns 256 adjacent bytes of every
+    // frame, the next tile is fetched while the current one is searched); segments that do not fill a tile go to the
+    // direct kernels below.
+    // <C, G, SS, warps per pipeline (= segments per tile), CTAs per SM, pipelines per CTA>: C column blocks of 16 bytes
+    // per warp (= seg / 16),
     // 4G words per lane; SS = stride of the stage-A sample words, which hold frames below 8P(3SS/2 + 1) (P = 4/C):
     // all real frames over the n-range of the variant
     const bool al16 = (reinterpret_cast<uintptr_t>(frames) % 16 == 0) && (m % 16 == 0);
-    const int64_t ntiles = nseg / 8;
-    if (al16 && path != 2 && n > 80 && ntiles > 0 && !g_median_direct) {
-      if (n <= 152) e = launch_median_sad_tma<4, 19, 6, 8, 2>(frames, n, m, ntiles, out, stream);
-      else if (n <= 232) e = launch_median_sad_tma<4, 29, 12, 8, 1>(frames, n, m, ntiles, out, stream);
-      else if (n <= 304) e = launch_median_sad_tma<4, 38, 19, 8, 1>(frames, n, m, ntiles, out, stream);
-      else if (n <= 464) e = launch_median_sad_tma<2, 29, 12, 8, 1>(frames, n, m, ntiles, out, stream);
-      else e = launch_median_sad_tma<2, 38, 19, 8, 1>(frames, n, m, ntiles, out, stream);
+    if (al16 && path != 2 && n > 80 && !g_median_direct) {
+      int64_t done = 0;
+      if (n <= 152) e = launch_median_sad_tma<4, 19, 6, 4, 1, 4>(frames, n, m, nseg, out, stream, &done);
+      else if (n <= 232) e = launch_median_sad_tma<4, 29, 12, 4, 1, 3>(frames, n, m, nseg, out, stream, &done);
+      else if (n <= 304) e = launch_median_sad_tma<4, 38, 19, 4, 1, 2>(frames, n, m, nseg, out, stream, &done);
+      else if (n <= 464) e = launch_median_sad_tma<2, 29, 12, 8, 1>(frames, n, m, nseg, out, stream, &done);
+      else e = launch_median_sad_tma<2, 38, 19, 8, 1>(frames, n, m, nseg, out, stream, &done);
       if (e == VU_OK) {
-        const int64_t done = ntiles * 8;
         frames += done * seg;
         out += done * seg;
         nseg -= done;
